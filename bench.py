@@ -2,7 +2,12 @@
 """bench.py -- Mrays/s of the ray-generation / intersection / shading hot path on N B200s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--gather peer|nccl]
+                  [--dump-outputs DIR]
   (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
+
+--dump-outputs DIR writes what the last timed step computed as .npy files: the frame (a fixed sample of 2 Mi pixels of a
+larger frame), or for pt_r2000_150 every accelerator's per-ray results.  Two builds run with the same arguments get the
+same seeded inputs and can be compared output for output.
 
 A step = one frame of the workload rendered by the hot path (ray generation -> accelerator traversal -> triangle /
 sphere / plane tests -> Whitted or Monte-Carlo shading -> framebuffer).  For N > 1 the frame is sharded over the ranks
@@ -189,6 +194,28 @@ def emit(line):
         os.write(_JSON_FD, data)
 
 
+DUMP_PIXELS = 1 << 21  # 2 Mi pixels: 24 MiB of float32 RGB + 16 MiB of float64 pixel indices
+
+
+def dump_outputs(out_dir, arrays, image=None):
+    """--dump-outputs: every array of `arrays` as out_dir/<name>.npy (float32 stays float32, anything else becomes
+    float64), and the frame `image` [H][W][3] float32 as image.npy.  A frame of more than DUMP_PIXELS pixels is
+    written as a fixed sample (seed 0) of that many pixels, [n][3], with their flat indices y * W + x, ascending,
+    as image_pixels.npy -- the same pixels for every run of the same frame size."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = dict(arrays)
+    if image is not None:
+        flat = np.ascontiguousarray(image, np.float32).reshape(-1, image.shape[-1])
+        if flat.shape[0] > DUMP_PIXELS:
+            idx = np.sort(np.random.default_rng(0).choice(flat.shape[0], DUMP_PIXELS, replace=False))
+            out["image"], out["image_pixels"] = flat[idx], idx
+        else:
+            out["image"] = image
+    for name, a in out.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float32 if a.dtype == np.float32 else np.float64))
+
+
 def run_reference(args, wl_name):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -258,16 +285,19 @@ def run_pt(args, wl_name):
     wl = WORKLOADS[wl_name]
     xy = pt_rays(wl["rays"])
     big = pt_rays(1 << 20, seed=6)  # the same workload at a size that fills the GPU
-    table = {}
-    steps = max(args.steps, 3)
+    table, last = {}, {}
+    steps = args.steps
     for alg in PT_ALGS:
         rtb200.perf_test(xy, wl["radius"], wl["angle"], wl["arch_seg"], wl["path_seg"], alg)  # warm-up (context, first launch)
         runs = [rtb200.perf_test(xy, wl["radius"], wl["angle"], wl["arch_seg"], wl["path_seg"], alg) for _ in range(steps)]
+        last.update({f"{alg}_{k}": runs[-1][k] for k in ("reached", "depth", "last_id", "last_pos")})
         b = rtb200.perf_test(big, wl["radius"], wl["angle"], wl["arch_seg"], wl["path_seg"], alg)
         table[alg] = {"trace_ms": float(np.mean([r["trace_ms"] for r in runs])), "build_ms": runs[-1]["build_ms"],
                       "preprocess_ms": runs[-1]["preprocess_ms"], "total_rays": int(runs[-1]["total_rays"]),
                       "published_trace_ms": PT_PUBLISHED_TRACE_MS[alg],
                       "at_1M_rays": {"trace_ms": b["trace_ms"], "Mrays/s": b["total_rays"] / b["trace_ms"] / 1e3, "total_rays": int(b["total_rays"])}}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     cpu = None
     if not args.no_cpu:
         try:
@@ -518,6 +548,8 @@ def run_b200(args, wl_name):
                 raise SystemExit("assembled multi-GPU frame differs from the single-GPU frame")
             gpu_image = assembled
         barrier()
+    if args.dump_outputs and rank == 0:  # the frame of the last timed step (--gather nccl: the unsharded frame on rank 0)
+        dump_outputs(args.dump_outputs, {}, gpu_image if gpu_image is not None else image.cpu().numpy())
 
     # ---- e2e: host buffers through the C ABI; scene H2D + render + the ASSEMBLED frame in one page-locked host buffer, per step
     e2e_steps = max(3, min(args.steps, 10))
@@ -734,7 +766,13 @@ def main():
     ap.add_argument("--mc-shard", default="auto", choices=["auto", "samples", "pixels"])
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 arm (--impl b200)")
+    sys.dont_write_bytecode = True  # the run leaves the tree as it found it (it may be read-only)
     # stdout carries exactly one JSON line: file descriptor 1 is pointed at stderr for the duration of the run
     # (NCCL prints its version banner to stdout whatever NCCL_DEBUG_FILE says) and emit() writes to the saved one
     global _JSON_FD
