@@ -57,13 +57,20 @@ typedef struct rtb_material {
 enum { RTB_PRIM_PLANE = 0,     /* Plane.cpp:3-34: v = normal xyz, position xyz, dist              */
        RTB_PRIM_SPHERE = 1,    /* Sphere.cpp:4-37: v = center xyz, radius                         */
        RTB_PRIM_TRIANGLES = 2, /* run of loose Triangle geometries (GeometrySet.cpp:33-86): first/count index loose_tri */
-       RTB_PRIM_TUNNEL = 3 };  /* the Tunnel geometry (Tunnel.cpp:1299-1309), traversed with `accel` */
+       RTB_PRIM_TUNNEL = 3,    /* the Tunnel geometry (Tunnel.cpp:1299-1309), traversed with `accel` */
+       /* A triangle MESH (a loaded model; no reference counterpart): the fields of a TRIANGLES run -- first/count index
+        * loose_tri (count >= 1), one material, triangle k has hit id base_id + k -- traversed through a bounding-volume
+        * hierarchy that rtb_scene_upload builds on the device (one per record, also when ranges overlap).  Contract: the
+        * nearest hit is the one the run of the same triangles returns -- the smallest t the reference's triangle test accepts, ties to the lowest k, compared with
+        * the earlier records by the same strict `<` -- except when the run's winning pair lies in the grazing band
+        * described in csrc/rtb_bvh.h (ray almost in the triangle's plane), where the reference's t is rounding noise.   */
+       RTB_PRIM_MESH = 4 };
 
 typedef struct rtb_prim {
     int32_t type;
     int32_t material; /* index into materials (ignored for TUNNEL: per-triangle) */
     int32_t base_id;  /* top-level geometry index of this record (of its first triangle for a run) */
-    int32_t first, count; /* TRIANGLES: range in loose_tri */
+    int32_t first, count; /* TRIANGLES, MESH: range in loose_tri */
     float v[7];
 } rtb_prim;           /* 48 bytes */
 
@@ -267,6 +274,22 @@ int rtb_scene_grid_hash(rtb_ctx *ctx, const rtb_scene *scene, uint64_t *hash, in
  * (min xyz, size xyz).  Either array may be NULL to query the counts first.                                            */
 int rtb_scene_kd_download(rtb_ctx *ctx, const rtb_scene *scene, rtb_kdnode *nodes, int64_t node_cap, uint32_t *leaf_tris,
                           int64_t ref_cap, int64_t counts[3], float box[6]);
+
+/* Bounding-volume hierarchy of an RTB_PRIM_MESH record (built on the device by rtb_scene_upload, csrc/rtb_build_bvh.cuh).
+ * A mesh of n triangles has max(n - 1, 1) inner nodes, node 0 is the root.  Each node holds the boxes of its two children
+ * (a child's box is the union of the boxes below it; a leaf's box is its triangle's box widened by the barycentric slack,
+ * csrc/rtb_bvh.h) and the two child links: c >= 0 is inner node c, c < 0 is the leaf at position ~c of the mesh's leaf
+ * order (one triangle per leaf; a one-triangle mesh has both links -1).  tri_order[p] = local index k (0 .. n - 1) of the
+ * triangle at leaf position p.                                                                                          */
+typedef struct rtb_bvhnode {
+    float lo[2][3], hi[2][3]; /* [child][axis] */
+    int32_t child[2];
+    int32_t pad_[2];
+} rtb_bvhnode;              /* 64 bytes */
+/* Inspection: the tree of the mesh record `mesh_index` (0 = the first MESH record in prims order).  counts = {inner nodes,
+ * triangles, depth (the root's children are at depth 1; leaves count)}.  nodes / tri_order may be NULL to query the counts. */
+int rtb_scene_mesh_download(rtb_ctx *ctx, const rtb_scene *scene, int32_t mesh_index, rtb_bvhnode *nodes, int64_t node_cap,
+                            uint32_t *tri_order, int64_t tri_cap, int64_t counts[3]);
 
 /* Replaces `int Render(GeometrySet&, PerspectiveCamera&, RenderSetting&, ProgressCallback)`
  * (reference MainWindow.cpp:251-303, the RenderProc of Scripts.h:11-12): ray generation,

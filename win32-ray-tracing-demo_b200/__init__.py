@@ -22,6 +22,7 @@ STAT_NAMES = ["n_top", "n_tris", "grid_x", "grid_y", "grid_z", "cells_nonempty",
               "cell_max", "kd_nodes", "kd_leaves", "kd_leaf_refs", "kd_max_depth"]
 LAYOUT_ROWMAJOR, LAYOUT_REFERENCE, LAYOUT_GLOBAL, OUTPUT_RGB8, OUTPUT_MOMENTS = 0, 1, 2, 4, 8
 IPC_HANDLE_BYTES = 64
+PRIM_PLANE, PRIM_SPHERE, PRIM_TRIANGLES, PRIM_TUNNEL, PRIM_MESH = 0, 1, 2, 3, 4  # rtb_prim.type
 
 
 class RtbError(RuntimeError):
@@ -43,6 +44,11 @@ class Prim(C.Structure):
 
 class KdNode(C.Structure):
     _fields_ = [("a", C.c_uint32), ("b", C.c_uint32)]
+
+
+class BvhNode(C.Structure):
+    """rtb_bvhnode: boxes lo/hi [child][axis] of the two children, child links (>= 0 inner node, < 0 leaf position ~c)."""
+    _fields_ = [("lo", (C.c_float * 3) * 2), ("hi", (C.c_float * 3) * 2), ("child", C.c_int32 * 2), ("pad_", C.c_int32 * 2)]
 
 
 class CellWord(C.Structure):
@@ -126,7 +132,7 @@ class Stats(C.Structure):
 ABI_SYMBOLS = ["rtb_init", "rtb_shutdown", "rtb_last_error", "rtb_abi_version", "rtb_shard_rows", "rtb_shard_width",
                "rtb_unshard_cols_device",
                "rtb_host_alloc", "rtb_host_free", "rtb_host_register", "rtb_host_unregister",
-               "rtb_scene_upload", "rtb_scene_free", "rtb_scene_device_bytes", "rtb_scene_upload_bytes", "rtb_scene_grid_hash", "rtb_scene_kd_download", "rtb_render",
+               "rtb_scene_upload", "rtb_scene_free", "rtb_scene_device_bytes", "rtb_scene_upload_bytes", "rtb_scene_grid_hash", "rtb_scene_kd_download", "rtb_scene_mesh_download", "rtb_render",
                "rtb_render_device", "rtb_unshard_device", "rtb_trace_primary", "rtb_intersect_rays", "rtb_bounce_rays",
                "rtb_selftest_pretest", "rtb_kd_validate", "rtb_forget_schedule", "rtb_set_progress", "rtb_multi_set_progress",
                "rtb_device_alloc", "rtb_device_free", "rtb_device_download", "rtb_ipc_export", "rtb_ipc_open", "rtb_ipc_close", "rtb_scatter_shard_device",
@@ -166,6 +172,7 @@ def cuda_lib():
         lib.rtb_scene_grid_hash.argtypes = [vp, vp, C.POINTER(C.c_uint64), C.POINTER(C.c_int64)]
         lib.rtb_scene_grid_hash.restype = C.c_int
         lib.rtb_scene_kd_download.argtypes = [vp, vp, vp, i64, vp, i64, C.POINTER(C.c_int64), C.POINTER(C.c_float)]
+        lib.rtb_scene_mesh_download.argtypes = [vp, vp, i32, vp, i64, vp, i64, C.POINTER(C.c_int64)]
         lib.rtb_render.argtypes = [vp, vp, C.POINTER(Camera), C.POINTER(RenderSetting), C.POINTER(Frame), vp,
                                    C.POINTER(Stats)]
         lib.rtb_render_device.argtypes = [vp, vp, C.POINTER(Camera), C.POINTER(RenderSetting), C.POINTER(Frame),
@@ -358,6 +365,12 @@ def set_exact_grid_binning(on):
 def set_kd_on_device(on):
     """Tunnels built from now on leave a KdTreeSAH accelerator to the device builder of rtb_scene_upload."""
     host_lib().rtbh_set_kd_on_device(1 if on else 0)
+
+
+def set_stl_as_mesh(on):
+    """Preset 3 built from now on loads its STL as one triangle mesh (GeometrySet::addStlMesh, RTB_PRIM_MESH) instead of
+    loose triangles: the same triangles and hit ids, traversed through a hierarchy built on the device."""
+    host_lib().rtbh_set_stl_as_mesh(1 if on else 0)
 
 
 def set_grid_on_device(on):
@@ -676,6 +689,21 @@ class DeviceScene:
                                                             counts, box), "rtb_scene_kd_download")
         return nodes, refs, int(counts[2]), np.array(list(box), np.float32)
 
+    def mesh_download(self, mesh_index=0):
+        """(lo [n][2][3], hi [n][2][3] float32, child [n][2] int32, tri_order [m] uint32, depth) of the hierarchy of the
+        mesh record `mesh_index` (include/rtb.h: rtb_bvhnode)."""
+        counts = (C.c_int64 * 3)()
+        lib = self.ctx._lib
+        self.ctx._check(lib.rtb_scene_mesh_download(self.ctx._h, self._h, mesh_index, None, 0, None, 0, counts), "rtb_scene_mesh_download")
+        nodes = (BvhNode * int(counts[0]))()
+        order = np.zeros(counts[1], np.uint32)
+        self.ctx._check(lib.rtb_scene_mesh_download(self.ctx._h, self._h, mesh_index, nodes, counts[0], order.ctypes.data, counts[1], counts),
+                        "rtb_scene_mesh_download")
+        raw = np.frombuffer(nodes, np.uint8).reshape(int(counts[0]), 64)
+        f = raw[:, :48].copy().view(np.float32).reshape(-1, 12)
+        child = raw[:, 48:56].copy().view(np.int32).reshape(-1, 2)
+        return f[:, :6].reshape(-1, 2, 3), f[:, 6:].reshape(-1, 2, 3), child, order, int(counts[2])
+
     def render(self, camera, setting, frame, out=None):
         """rtb_render with HOST buffers; returns (rows x width x 3 float32 | reference-order array, stats)."""
         rows = shard_rows(frame)
@@ -719,3 +747,38 @@ class DeviceScene:
                                                          ht.ctypes.data, pos.ctypes.data, nrm.ctypes.data),
                         "rtb_intersect_rays")
         return hid, ht, pos, nrm
+
+
+# ---- synthetic models -------------------------------------------------------------------------
+def torus_triangles(n_triangles, seed=0, major=15.0, minor=6.0, center=(0.0, 16.0, 0.0)):
+    """[n][12] float32 facets (normal, a, b, c: the binary STL facet order) of a closed torus tessellated into about
+    n_triangles triangles (2 per grid quad, ring:tube = 2:1), every grid vertex displaced by a seeded jitter of 2 % of
+    the tube's grid spacing.  Default size and place: inside the smallpt box of preset 3 once its STL offset is added."""
+    nv = max(3, int(round(np.sqrt(n_triangles / 4.0))))
+    nu = max(3, int(round(n_triangles / (2.0 * nv))))
+    rng = np.random.default_rng(seed)
+    u = (np.arange(nu) / nu * 2 * np.pi)[:, None]
+    v = (np.arange(nv) / nv * 2 * np.pi)[None, :]
+    rr = minor * (1 + 0.02 * (2 * np.pi / nv) * rng.uniform(-1, 1, (nu, nv)))
+    x = (major + rr * np.cos(v)) * np.cos(u) + center[0]
+    y = rr * np.sin(v) + center[1]
+    z = (major + rr * np.cos(v)) * np.sin(u) + center[2]
+    p = np.stack([x, y, z], -1).astype(np.float32)
+    i, j = np.meshgrid(np.arange(nu), np.arange(nv), indexing="ij")
+    i1, j1 = (i + 1) % nu, (j + 1) % nv
+    a, b, c, d = p[i, j], p[i1, j], p[i1, j1], p[i, j1]
+    t = np.concatenate([np.stack([a, b, c], -2).reshape(-1, 3, 3), np.stack([a, c, d], -2).reshape(-1, 3, 3)])
+    n = np.cross(t[:, 1] - t[:, 0], t[:, 2] - t[:, 0])
+    n /= np.maximum(np.linalg.norm(n, axis=1, keepdims=True), 1e-30)
+    return np.concatenate([n.astype(np.float32), t.reshape(-1, 9)], 1).astype(np.float32)
+
+
+def write_stl(path, facets):
+    """Binary STL of [n][12] float32 facets (normal, a, b, c), the format GeometrySet::addStlFile / addStlMesh read."""
+    facets = np.ascontiguousarray(facets, np.float32).reshape(-1, 12)
+    rec = np.zeros(len(facets), np.dtype([("f", "<f4", 12), ("attr", "<u2")]))
+    rec["f"] = facets
+    with open(path, "wb") as fh:
+        fh.write(b"\0" * 80)
+        fh.write(np.uint32(len(facets)).tobytes())
+        fh.write(rec.tobytes())

@@ -20,6 +20,7 @@
 #include "rtb_misc.cuh"
 #include "rtb_build_grid.cuh"
 #include "rtb_build_kd.cuh"
+#include "rtb_build_bvh.cuh"
 
 #ifndef RTB_SPLIT_MAX_TILES
 #define RTB_SPLIT_MAX_TILES 200000 // shards up to 6.4 Mpixel (half a 4K frame) count as "small": their latency-critical tiles go
@@ -254,6 +255,8 @@ struct rtb_scene
     int64_t h2d_bytes = 0; // bytes the upload copied from host memory (the rest is produced on the device)
     bool has_refractive = false;
     bool has_tunnel = false;
+    bool has_mesh = false;   // RTB_PRIM_MESH records: the MESH kernel instantiations, no tunnel tiers
+    std::vector<int> mesh_prims; // prims indices of the MESH records (rtb_scene_mesh_download)
     cudaEvent_t last_use = nullptr; // recorded after every launch that reads the scene
     cudaEvent_t ready = nullptr;    // recorded on ctx->stream behind the upload copies
     bool direct_sources = false;    // some copies read the caller's page-locked arrays: rtb_scene_free waits for `ready`
@@ -1158,6 +1161,74 @@ static size_t stagedBytesBound(const rtb_flat_scene *f)
     return t + 4096;
 }
 
+// Hierarchies of the MESH records (rtb_build_bvh.cuh) from the raw loose records on the device.  Every record gets its own
+// slice of the three arrays (DScene::mesh_base: the mesh triangles of the records before it), so records whose loose ranges
+// overlap each have their own tree; a mesh of n triangles uses max(n - 1, 1) <= n node slots (the spare one stays zero).
+static int buildMeshesOnDevice(rtb_ctx *ctx, rtb_scene *s, const float *d_raw)
+{
+    DScene &d = s->d;
+    cudaStream_t st = ctx->stream;
+    int rc;
+    size_t total = 0;
+    for (int i : s->mesh_prims)
+    {
+        d.mesh_base[i] = (int)total;
+        total += (size_t)d.prims[i].count;
+    }
+    if (total > 0x7fffffffull) return fail(ctx, RTB_ERR_UNSUPPORTED, "rtb_scene_upload: more than 2^31 - 1 mesh triangles in all");
+    rtb_bvhnode *nodes = nullptr;
+    float4 *tris = nullptr;
+    uint32_t *order = nullptr;
+    if ((rc = deviceArray(ctx, s, total, &nodes, true)) != RTB_OK) return rc;
+    if ((rc = deviceArray(ctx, s, 3 * total, &tris, true)) != RTB_OK) return rc;
+    if ((rc = deviceArray(ctx, s, total, &order, true)) != RTB_OK) return rc;
+    CUDA_TRY(ctx, cudaMemsetAsync(nodes, 0, total * sizeof(rtb_bvhnode), st));
+    d.mesh_nodes = reinterpret_cast<const float4 *>(nodes);
+    d.mesh_tris = tris;
+    d.mesh_order = order;
+    std::vector<void *> temps;
+    auto temp = [&](size_t bytes, void **p) { cudaError_t e = cudaMallocAsync(p, bytes ? bytes : 1, st); if (e == cudaSuccess) temps.push_back(*p); return e; };
+    auto cleanup = [&]() { for (void *p : temps) cudaFreeAsync(p, st); };
+#define MESH_TRY(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { cleanup(); return fail(ctx, RTB_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } } while (0)
+    size_t maxN = 0;
+    for (int i : s->mesh_prims) maxN = std::max(maxN, (size_t)d.prims[i].count);
+    unsigned int *d_bounds = nullptr, *d_arrivals = nullptr;
+    unsigned long long *d_keys = nullptr, *d_sorted = nullptr;
+    int *d_parent = nullptr;
+    void *d_tmp = nullptr;
+    size_t tmpBytes = 0;
+    MESH_TRY(cub::DeviceRadixSort::SortKeys(nullptr, tmpBytes, d_keys, d_sorted, (int)maxN, 0, 62, st));
+    MESH_TRY(temp(6 * sizeof(unsigned int), (void **)&d_bounds));
+    MESH_TRY(temp(maxN * sizeof(unsigned int), (void **)&d_arrivals));
+    MESH_TRY(temp(maxN * sizeof(unsigned long long), (void **)&d_keys));
+    MESH_TRY(temp(maxN * sizeof(unsigned long long), (void **)&d_sorted));
+    MESH_TRY(temp(2 * maxN * sizeof(int), (void **)&d_parent));
+    MESH_TRY(temp(tmpBytes, &d_tmp));
+    for (int i : s->mesh_prims)
+    {
+        const rtb_prim &P = d.prims[i];
+        const int n = P.count;
+        const unsigned int tb = 256, nb = (unsigned int)((n + tb - 1) / tb);
+        const float *raw = d_raw + 12ull * (unsigned int)P.first;
+        MESH_TRY(cudaMemsetAsync(d_bounds, 0xff, 3 * sizeof(unsigned int), st));
+        MESH_TRY(cudaMemsetAsync(d_bounds + 3, 0, 3 * sizeof(unsigned int), st));
+        MESH_TRY(cudaMemsetAsync(d_arrivals, 0, (size_t)n * sizeof(unsigned int), st));
+        k_bvh_bounds<<<nb, tb, 0, st>>>(raw, n, d_bounds);
+        k_bvh_keys<<<nb, tb, 0, st>>>(raw, n, d_bounds, d_keys);
+        size_t need = tmpBytes;
+        MESH_TRY(cub::DeviceRadixSort::SortKeys(d_tmp, need, d_keys, d_sorted, n, 0, 62, st));
+        const size_t base = (size_t)d.mesh_base[i];
+        rtb_bvhnode *mn = nodes + base;
+        if (n > 1) k_bvh_hierarchy<<<(unsigned int)((n - 1 + tb - 1) / tb), tb, 0, st>>>(d_sorted, n, mn, d_parent, d_parent + maxN);
+        k_bvh_boxes<<<nb, tb, 0, st>>>(raw, d_sorted, n, mn, d_parent, d_parent + maxN, d_arrivals);
+        k_bvh_leaves<<<nb, tb, 0, st>>>(d.loose + 3ull * (unsigned int)P.first, d_sorted, n, tris + 3 * base, order + base);
+        MESH_TRY(cudaGetLastError());
+    }
+#undef MESH_TRY
+    cleanup();
+    return RTB_OK;
+}
+
 static int sceneUpload(rtb_ctx *ctx, const rtb_flat_scene *f, rtb_scene **out, bool validate);
 
 extern "C" int rtb_scene_upload(rtb_ctx *ctx, const rtb_flat_scene *f, rtb_scene **out) { return sceneUpload(ctx, f, out, true); }
@@ -1191,14 +1262,17 @@ static int sceneUpload(rtb_ctx *ctx, const rtb_flat_scene *f, rtb_scene **out, b
     {
         const rtb_prim &p = f->prims[i];
         d.prims[i] = p;
-        bool ok = p.type >= RTB_PRIM_PLANE && p.type <= RTB_PRIM_TUNNEL;
+        bool ok = p.type >= RTB_PRIM_PLANE && p.type <= RTB_PRIM_MESH;
         if (p.type != RTB_PRIM_TUNNEL) ok = ok && p.material >= 0 && p.material < f->n_materials;
-        if (p.type == RTB_PRIM_TRIANGLES) ok = ok && p.first >= 0 && p.count >= 0 && p.first + p.count <= f->n_loose && f->loose_tri;
+        if (p.type == RTB_PRIM_TRIANGLES || p.type == RTB_PRIM_MESH)
+            ok = ok && p.first >= 0 && p.count >= 0 && (int64_t)p.first + p.count <= f->n_loose && f->loose_tri;
+        if (p.type == RTB_PRIM_MESH) { ok = ok && p.count >= 1; s->mesh_prims.push_back(i); }
         if (p.type == RTB_PRIM_TUNNEL) tunnels++;
         if (!ok) { rtb_scene_free(ctx, s); return fail(ctx, RTB_ERR_INVALID, "rtb_scene_upload: bad top-level record " + std::to_string(i)); }
     }
     if (tunnels > 1) { rtb_scene_free(ctx, s); return fail(ctx, RTB_ERR_UNSUPPORTED, "rtb_scene_upload: one tunnel per scene"); }
     s->has_tunnel = tunnels == 1;
+    s->has_mesh = !s->mesh_prims.empty();
     for (int i = 0; i < f->n_materials; i++)
     {
         d.mats[i] = f->materials[i];
@@ -1229,7 +1303,17 @@ static int sceneUpload(rtb_ctx *ctx, const rtb_flat_scene *f, rtb_scene **out, b
     // every stream is packed / copied into the page-locked staging ring and leaves with an asynchronous copy:
     // no intermediate synchronisation, the upload is ordered before the renders on ctx->stream
     const size_t nLoose = f->loose_tri ? (size_t)f->n_loose : 0;
-    if ((rc = uploadTriangles(ctx, s, f->loose_tri, nLoose, &d.loose, nullptr)) != RTB_OK) return bail(rc);
+    {
+        float *d_rawLoose = nullptr; // kept for the mesh builds
+        if ((rc = uploadTriangles(ctx, s, f->loose_tri, nLoose, &d.loose, nullptr, s->has_mesh ? &d_rawLoose : nullptr)) != RTB_OK) return bail(rc);
+        if (s->has_mesh)
+        {
+            rc = buildMeshesOnDevice(ctx, s, d_rawLoose);
+            cudaFreeAsync(d_rawLoose, ctx->stream);
+            if (rc != RTB_OK) return bail(rc);
+            laps.lap("mesh hierarchies");
+        }
+    }
 
     if (s->has_tunnel)
     {
@@ -1434,6 +1518,53 @@ extern "C" int rtb_scene_kd_download(rtb_ctx *ctx, const rtb_scene *s, rtb_kdnod
     return RTB_OK;
 }
 
+extern "C" int rtb_scene_mesh_download(rtb_ctx *ctx, const rtb_scene *s, int32_t mesh_index, rtb_bvhnode *nodes, int64_t node_cap,
+                                       uint32_t *tri_order, int64_t tri_cap, int64_t counts[3])
+{
+    if (!ctx || !s) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_download: null argument");
+    if (mesh_index < 0 || mesh_index >= (int32_t)s->mesh_prims.size())
+        return fail(ctx, RTB_ERR_UNSUPPORTED, "rtb_scene_mesh_download: the scene has no such mesh record");
+    const rtb_prim &P = s->d.prims[s->mesh_prims[(size_t)mesh_index]];
+    const int64_t nNodes = P.count > 1 ? P.count - 1 : 1;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    std::vector<rtb_bvhnode> all((size_t)nNodes);
+    const size_t base = (size_t)s->d.mesh_base[s->mesh_prims[(size_t)mesh_index]];
+    CUDA_TRY(ctx, cudaMemcpyAsync(all.data(), s->d.mesh_nodes + 4 * base, (size_t)nNodes * sizeof(rtb_bvhnode),
+                                  cudaMemcpyDeviceToHost, ctx->stream));
+    if (tri_order)
+    {
+        if (tri_cap < P.count) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_download: order buffer too small");
+        CUDA_TRY(ctx, cudaMemcpyAsync(tri_order, s->d.mesh_order + base, (size_t)P.count * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    if (nodes)
+    {
+        if (node_cap < nNodes) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_download: node buffer too small");
+        memcpy(nodes, all.data(), (size_t)nNodes * sizeof(rtb_bvhnode));
+    }
+    if (counts)
+    { // depth by an explicit walk; a link outside the node array ends the walk as an error
+        int64_t depth = 0;
+        std::vector<std::pair<int32_t, int64_t>> stack{{0, 0}};
+        int64_t visited = 0;
+        while (!stack.empty())
+        {
+            const auto [node, dep] = stack.back();
+            stack.pop_back();
+            if (++visited > nNodes) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_download: malformed tree");
+            for (int c = 0; c < (P.count > 1 ? 2 : 1); c++)
+            {
+                const int32_t ch = all[(size_t)node].child[c];
+                if (ch < 0) depth = std::max(depth, dep + 1);
+                else if (ch < nNodes) stack.push_back({ch, dep + 1});
+                else return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_download: malformed tree");
+            }
+        }
+        counts[0] = nNodes; counts[1] = P.count; counts[2] = depth;
+    }
+    return RTB_OK;
+}
+
 // ---- render -----------------------------------------------------------------------------------
 static int makeFrame(rtb_ctx *ctx, const rtb_scene *scene, const rtb_camera *cam, const rtb_render_setting *setting,
                      const rtb_frame *frame, FrameParams &F)
@@ -1522,9 +1653,10 @@ static int launchRender(rtb_ctx *ctx, const rtb_scene *scene, FrameParams &F, bo
     const bool kd_accel = accel == RTB_ACCEL_KD_MEDIAN || accel == RTB_ACCEL_KD_SAH;
     F.skip_heavy = 0;
     F.record_cost = 1;
-    auto L = [&](const FrameParams &P, dim3 g, cudaStream_t st) { Launch l; l.S = &scene->d; l.F = &P; l.out = out; l.counters = counters; l.grid = g; l.stream = st; l.count = count; return l; };
+    auto L = [&](const FrameParams &P, dim3 g, cudaStream_t st) { Launch l; l.S = &scene->d; l.F = &P; l.out = out; l.counters = counters; l.grid = g; l.stream = st; l.count = count; l.mesh = scene->has_mesh; return l; };
     if (F.setting.enable_monte_carlo) launchMonteCarlo(L(F, grid, stream));
     else if (scene->has_refractive) launchTree(L(F, grid, stream));
+    else if (scene->has_mesh) launchChain(L(F, grid, stream)); // the latency tiers have no mesh walk
     else if (resumable && scene->has_tunnel && (kd_accel || grid_accel) && F.order && ctx->tiers_ok)
     { // A tile order is known.  Three kernels share the frame, all launched at once:
       //   order[0 .. n_wide)         the very heaviest tiles: one warp per pixel        (side stream, high priority)
@@ -2294,7 +2426,8 @@ extern "C" int rtb_trace_primary(rtb_ctx *ctx, const rtb_scene *scene, const rtb
     if (seq_hash) CUDA_TRY(ctx, d_hash.alloc(n));
     if (seq_buf) CUDA_TRY(ctx, d_buf.alloc(n * seq_cap));
     const dim3 grid((unsigned int)((F.n_tiles + RTB_CTA_THREADS / 32 - 1) / (RTB_CTA_THREADS / 32)));
-    k_trace_primary<<<grid, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, F, d_id.p, d_t.p, d_len.p, d_hash.p, d_buf.p, seq_cap);
+    if (scene->has_mesh) k_trace_primary<true><<<grid, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, F, d_id.p, d_t.p, d_len.p, d_hash.p, d_buf.p, seq_cap);
+    else k_trace_primary<<<grid, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, F, d_id.p, d_t.p, d_len.p, d_hash.p, d_buf.p, seq_cap);
     CUDA_TRY(ctx, cudaGetLastError());
     if (hit_id) CUDA_TRY(ctx, cudaMemcpyAsync(hit_id, d_id.p, n * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     if (hit_t) CUDA_TRY(ctx, cudaMemcpyAsync(hit_t, d_t.p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
@@ -2320,7 +2453,8 @@ extern "C" int rtb_intersect_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t 
     if (position) CUDA_TRY(ctx, d_pos.alloc((size_t)n * 3));
     if (normal) CUDA_TRY(ctx, d_nrm.alloc((size_t)n * 3));
     const unsigned int blocks = (unsigned int)((n + RTB_CTA_THREADS - 1) / RTB_CTA_THREADS);
-    k_intersect_rays<<<blocks, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, (long long)n, d_rays.p, d_id.p, d_t.p, d_pos.p, d_nrm.p);
+    if (scene->has_mesh) k_intersect_rays<true><<<blocks, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, (long long)n, d_rays.p, d_id.p, d_t.p, d_pos.p, d_nrm.p);
+    else k_intersect_rays<<<blocks, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, (long long)n, d_rays.p, d_id.p, d_t.p, d_pos.p, d_nrm.p);
     CUDA_TRY(ctx, cudaGetLastError());
     if (hit_id) CUDA_TRY(ctx, cudaMemcpyAsync(hit_id, d_id.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     if (hit_t) CUDA_TRY(ctx, cudaMemcpyAsync(hit_t, d_t.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
@@ -2352,7 +2486,7 @@ extern "C" int rtb_bounce_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, 
     const int accel = scene->d.accel;
     const bool walkable = scene->has_tunnel && (accel == RTB_ACCEL_REGULAR_GRID || accel == RTB_ACCEL_FLAT_GRID || accel == RTB_ACCEL_KD_MEDIAN || accel == RTB_ACCEL_KD_SAH);
     static const long long wideMax = (long long)tunable("RTB_BOUNCE_WIDE_MAX", 148 * 64 * 2); // up to two warps per resident warp slot
-    const bool wide = walkable && n <= wideMax;
+    const bool wide = walkable && n <= wideMax && !scene->has_mesh; // the warp-per-ray walk has no mesh walk
     // one lane per ray: the lanes pull rays from a queue (Counters::steps doubles as its head), the grid fills the device once
     const long long resident = 148ll * 16 * RTB_CTA_THREADS;
     const long long threads = wide ? n * 32 : (n < resident ? n : resident);
@@ -2360,6 +2494,9 @@ extern "C" int rtb_bounce_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, 
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[1], ctx->stream));
     if (wide) k_bounce_rays<true><<<blocks, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, (long long)n, d_rays.p, max_depth, d_ok.p, d_depth.p, d_id.p,
                                                                              d_pos.p, &ctx->d_counters->rays, &ctx->d_counters->steps);
+    else if (scene->has_mesh)
+        k_bounce_rays<false, true><<<blocks, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, (long long)n, d_rays.p, max_depth, d_ok.p, d_depth.p, d_id.p,
+                                                                              d_pos.p, &ctx->d_counters->rays, &ctx->d_counters->steps);
     else k_bounce_rays<false><<<blocks, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, (long long)n, d_rays.p, max_depth, d_ok.p, d_depth.p, d_id.p,
                                                                            d_pos.p, &ctx->d_counters->rays, &ctx->d_counters->steps);
     CUDA_TRY(ctx, cudaGetLastError());

@@ -1,0 +1,160 @@
+// rtb_build_bvh.cuh -- device build of the hierarchy of an RTB_PRIM_MESH record (include/rtb.h: rtb_bvhnode), from the raw
+// loose-triangle records already on the device.  A linear BVH (Karras, "Maximizing parallelism in the construction of BVHs,
+// octrees, and k-d trees", HPG 2012):
+//   1. centroid bounds (float min / max through order-preserving integer atomics: exact, order-independent);
+//   2. 62-bit keys: the 30-bit Morton code of the centroid, then the local index (32 bits) -- all keys differ, so every
+//      inner node splits on a strictly lower bit than its parent and the depth of inner nodes is at most 62;
+//   3. radix sort of the keys;
+//   4. hierarchy: inner node i covers a key range found from the common-prefix lengths of its neighbours;
+//   5. boxes bottom-up: the second thread to reach a node takes the union of its two child boxes (float min / max only);
+//   6. the triangle records (exact stream) copied into leaf order, with the local index of each leaf.
+// Every step is a deterministic function of the input: two builds of the same mesh are byte-identical.
+#pragma once
+#include <cub/cub.cuh>
+#include "rtb_bvh.h"
+
+namespace rtb {
+
+__device__ __forceinline__ unsigned int orderedBits(float f)
+{
+    const unsigned int u = __float_as_uint(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float orderedFloat(unsigned int u) { return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u); }
+
+__device__ __forceinline__ void triCentroid(const float *raw, unsigned int k, float c[3])
+{
+    const float *v = raw + 12ull * k;
+    for (int i = 0; i < 3; i++) c[i] = (v[i] + v[3 + i] + v[6 + i]) * (1.0f / 3.0f);
+}
+
+// bounds[0..2] = ordered min, bounds[3..5] = ordered max of the centroids (initialised to 0xffffffff / 0)
+__global__ void k_bvh_bounds(const float *__restrict__ raw, int n, unsigned int *__restrict__ bounds)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    float c[3];
+    triCentroid(raw, (unsigned int)k, c);
+    for (int i = 0; i < 3; i++)
+    {
+        atomicMin(bounds + i, orderedBits(c[i]));
+        atomicMax(bounds + 3 + i, orderedBits(c[i]));
+    }
+}
+
+__device__ __forceinline__ unsigned long long spread10(unsigned int v)
+{
+    unsigned long long x = v & 0x3ffu;
+    x = (x | (x << 16)) & 0x030000FFull;
+    x = (x | (x << 8)) & 0x0300F00Full;
+    x = (x | (x << 4)) & 0x030C30C3ull;
+    x = (x | (x << 2)) & 0x09249249ull;
+    return x;
+}
+
+__global__ void k_bvh_keys(const float *__restrict__ raw, int n, const unsigned int *__restrict__ bounds, unsigned long long *__restrict__ keys)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    float c[3];
+    triCentroid(raw, (unsigned int)k, c);
+    unsigned long long m = 0;
+    for (int i = 0; i < 3; i++)
+    {
+        const float lo = orderedFloat(bounds[i]), hi = orderedFloat(bounds[3 + i]);
+        const float ext = hi - lo;
+        float q = ext > 0.0f ? (c[i] - lo) / ext * 1024.0f : 0.0f;
+        q = (q >= 0.0f) ? fminf(q, 1023.0f) : 0.0f; // NaN -> 0
+        m |= spread10((unsigned int)q) << (2 - i);
+    }
+    keys[k] = (m << 32) | (unsigned int)k;
+}
+
+__device__ __forceinline__ int commonPrefix(const unsigned long long *keys, int n, int i, int j)
+{
+    if (j < 0 || j >= n) return -1;
+    return __clzll(keys[i] ^ keys[j]);
+}
+
+// inner node i of n - 1 (n >= 2); parent links: 2 * parent + side, for inner nodes and leaves
+__global__ void k_bvh_hierarchy(const unsigned long long *__restrict__ keys, int n, rtb_bvhnode *__restrict__ nodes,
+                                int *__restrict__ parent_inner, int *__restrict__ parent_leaf)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n - 1) return;
+    const int d = (commonPrefix(keys, n, i, i + 1) - commonPrefix(keys, n, i, i - 1)) >= 0 ? 1 : -1;
+    const int dmin = commonPrefix(keys, n, i, i - d);
+    int lmax = 2;
+    while (commonPrefix(keys, n, i, i + lmax * d) > dmin) lmax *= 2;
+    int l = 0;
+    for (int t = lmax / 2; t >= 1; t /= 2)
+        if (commonPrefix(keys, n, i, i + (l + t) * d) > dmin) l += t;
+    const int j = i + l * d;
+    const int dnode = commonPrefix(keys, n, i, j);
+    int s = 0, t = l;
+    do
+    {
+        t = (t + 1) >> 1;
+        if (commonPrefix(keys, n, i, i + (s + t) * d) > dnode) s += t;
+    } while (t > 1);
+    const int split = i + s * d + (d < 0 ? -1 : 0);
+    const int first = i < j ? i : j, last = i < j ? j : i;
+    const int left = (first == split) ? ~split : split;
+    const int right = (last == split + 1) ? ~(split + 1) : split + 1;
+    nodes[i].child[0] = left;
+    nodes[i].child[1] = right;
+    nodes[i].pad_[0] = nodes[i].pad_[1] = 0;
+    if (left < 0) parent_leaf[~left] = 2 * i; else parent_inner[left] = 2 * i;
+    if (right < 0) parent_leaf[~right] = 2 * i + 1; else parent_inner[right] = 2 * i + 1;
+}
+
+// one thread per leaf position p: leaf box into its parent's slot, then up while this thread is the second to arrive
+__global__ void k_bvh_boxes(const float *__restrict__ raw, const unsigned long long *__restrict__ keys, int n,
+                            rtb_bvhnode *__restrict__ nodes, const int *__restrict__ parent_inner,
+                            const int *__restrict__ parent_leaf, unsigned int *__restrict__ arrivals)
+{
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n) return;
+    float lo[3], hi[3];
+    rtb_bvh::leafBox(raw + 12ull * (unsigned int)(keys[p] & 0xffffffffull), lo, hi);
+    if (n == 1)
+    { // a single leaf: both links of the root point at it
+        for (int c = 0; c < 2; c++)
+        {
+            for (int a = 0; a < 3; a++) { nodes[0].lo[c][a] = lo[a]; nodes[0].hi[c][a] = hi[a]; }
+            nodes[0].child[c] = ~0;
+        }
+        nodes[0].pad_[0] = nodes[0].pad_[1] = 0;
+        return;
+    }
+    int slot = parent_leaf[p];
+    while (true)
+    {
+        const int node = slot >> 1, side = slot & 1;
+        for (int a = 0; a < 3; a++) { nodes[node].lo[side][a] = lo[a]; nodes[node].hi[side][a] = hi[a]; }
+        __threadfence();
+        if (atomicAdd(arrivals + node, 1u) == 0u) return; // the sibling is still on its way: it continues
+        __threadfence();
+        const float *q = reinterpret_cast<const float *>(nodes + node);
+        for (int a = 0; a < 3; a++)
+        {
+            lo[a] = fminf(__ldcg(q + a), __ldcg(q + 3 + a));
+            hi[a] = fmaxf(__ldcg(q + 6 + a), __ldcg(q + 9 + a));
+        }
+        if (node == 0) return;
+        slot = parent_inner[node];
+    }
+}
+
+// triangle records in leaf order, and the local index of each leaf
+__global__ void k_bvh_leaves(const float4 *__restrict__ exact, const unsigned long long *__restrict__ keys, int n,
+                             float4 *__restrict__ leaf_tris, uint32_t *__restrict__ leaf_order)
+{
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n) return;
+    const unsigned int k = (unsigned int)(keys[p] & 0xffffffffull);
+    for (int j = 0; j < 3; j++) leaf_tris[3ull * p + j] = exact[3ull * k + j];
+    leaf_order[p] = k;
+}
+
+} // namespace rtb

@@ -14,6 +14,7 @@
 #include <float.h>
 #include "../../include/rtb.h"
 #include "rtb_pretest.h"
+#include "rtb_bvh.h"
 
 #define RTB_MAX_INLINE_PRIMS 16
 #define RTB_MAX_INLINE_MATS 16
@@ -107,6 +108,14 @@ struct DScene
     const uint8_t *cx_status;
     const short *cx_range;
     const uint16_t *cx_order;
+    // RTB_PRIM_MESH (rtb_build_bvh.cuh): every mesh record has its own slice of the three arrays, starting at
+    // mesh_base[record index] (the mesh triangles of the records before it): its inner nodes at mesh_nodes[base ..]
+    // (4 float4 each, the rtb_bvhnode layout), its triangles in leaf order at mesh_tris[base ..] (the exact stream's
+    // format) and their local indices at mesh_order[base ..]
+    const float4 *mesh_nodes;
+    const float4 *mesh_tris;
+    const uint32_t *mesh_order;
+    int mesh_base[RTB_MAX_INLINE_PRIMS];
 };
 
 // Ray::context (reference Ray.h:11-16, RayContext.h:5-13): written by the convex accelerator, copied to the
@@ -657,6 +666,49 @@ __device__ bool convexIntersect(const DScene &S, const Ray &ray, RayCtx &ctx, in
 }
 
 // ---------------------------------------------------------------------------------------------
+// Triangle mesh (RTB_PRIM_MESH): the hierarchy of rtb_build_bvh.cuh, nodes skipped by the test of rtb_bvh.h.  Nearest
+// accepted (t, k) in lexicographic order; `bestT` comes in as the nearest hit of the earlier records and `bestK` as -1, so
+// the mesh replaces it only with a strictly smaller t, as the run's `t < minDistance` does.  Visit order changes nothing.
+// ---------------------------------------------------------------------------------------------
+template <class Probe>
+__device__ bool meshIntersect(const DScene &S, unsigned int base, const Ray &ray, float &bestT, int &bestK, V3 &nOut, Probe &pr)
+{
+    const rtb_bvh::Ray R = rtb_bvh::makeRay(ray.o.x, ray.o.y, ray.o.z, ray.d.x, ray.d.y, ray.d.z);
+    const float4 *nodes = S.mesh_nodes + 4ull * base;
+    int stack[RTB_BVH_STACK];
+    int sp = 0, node = 0;
+    bool found = false;
+    auto leaf = [&](int pos) {
+        const TriData T = loadTri(S.mesh_tris, base + (unsigned int)pos);
+        pr.tri();
+        float t;
+        if (!triIntersect(T, ray, t)) return;
+        const int k = (int)__ldg(S.mesh_order + base + pos);
+        if (t < bestT || (t == bestT && k < bestK)) { bestT = t; bestK = k; nOut = triNormal(T); found = true; }
+    };
+    while (true)
+    {
+        pr.step(node);
+        const float4 *q = nodes + 4ull * (unsigned int)node;
+        const float4 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2), q3 = __ldg(q + 3);
+        const float lo0[3] = {q0.x, q0.y, q0.z}, lo1[3] = {q0.w, q1.x, q1.y};
+        const float hi0[3] = {q1.z, q1.w, q2.x}, hi1[3] = {q2.y, q2.z, q2.w};
+        const int c0 = __float_as_int(q3.x), c1 = __float_as_int(q3.y);
+        const bool h0 = rtb_bvh::nodeHit(R, lo0, hi0, bestT);
+        const bool h1 = c1 != c0 && rtb_bvh::nodeHit(R, lo1, hi1, bestT); // a one-triangle mesh links its leaf twice
+        if (h0 && c0 < 0) leaf(~c0);
+        if (h1 && c1 < 0) leaf(~c1);
+        const bool in0 = h0 && c0 >= 0, in1 = h1 && c1 >= 0;
+        if (in0 && in1) { stack[sp++] = c1; node = c0; }
+        else if (in0) node = c0;
+        else if (in1) node = c1;
+        else if (sp > 0) node = stack[--sp];
+        else break;
+    }
+    return found;
+}
+
+// ---------------------------------------------------------------------------------------------
 // GeometrySet::intersect -- reference GeometrySet.cpp:95-110 (+ Plane.cpp:9-34, Sphere.cpp:10-37)
 // ---------------------------------------------------------------------------------------------
 struct Hit { int id; int mat; int prim_type; float t; V3 pos, n; };
@@ -664,7 +716,8 @@ struct Hit { int id; int mat; int prim_type; float t; V3 pos, n; };
 // `tunnel(tri, t, n)` supplies the result of the TUNNEL geometry (a traversal, or a result computed
 // earlier by the resumable traversal of rtb_chain_sm.cuh); everything else is evaluated here in
 // insertion order with the reference's strict `<`.
-template <class Probe, class TunnelFn>
+// MESH = false: scenes without RTB_PRIM_MESH records (the kernels every other scene runs are compiled without the mesh walk)
+template <bool MESH = false, class Probe, class TunnelFn>
 __device__ __forceinline__ bool sceneIntersectWith(const DScene &S, const Ray &ray, Hit &best, Probe &pr, TunnelFn tunnel)
 {
     float minDistance = FLT_MAX;
@@ -724,6 +777,15 @@ __device__ __forceinline__ bool sceneIntersectWith(const DScene &S, const Ray &r
                 }
             }
         }
+        else if (MESH && P.type == RTB_PRIM_MESH)
+        {
+            int k = -1;
+            V3 n;
+            if (meshIntersect(S, (unsigned int)S.mesh_base[i], ray, minDistance, k, n, pr))
+            {
+                best.id = P.base_id + k; best.mat = P.material; best.n = n; best.prim_type = RTB_PRIM_MESH;
+            }
+        }
         else
         {
             int tri = -1;
@@ -743,10 +805,10 @@ __device__ __forceinline__ bool sceneIntersectWith(const DScene &S, const Ray &r
     return true;
 }
 
-template <class Probe>
+template <bool MESH = false, class Probe>
 __device__ bool sceneIntersect(const DScene &S, const Ray &ray, Hit &best, Probe &pr, RayCtx &ctx)
 {
-    return sceneIntersectWith(S, ray, best, pr, [&](int &tri, float &t, V3 &n) {
+    return sceneIntersectWith<MESH>(S, ray, best, pr, [&](int &tri, float &t, V3 &n) {
         if (S.accel == RTB_ACCEL_REGULAR_GRID || S.accel == RTB_ACCEL_FLAT_GRID) return gridIntersect<false>(S, ray, tri, t, n, pr);
         if (S.accel == RTB_ACCEL_KD_MEDIAN || S.accel == RTB_ACCEL_KD_SAH) return kdIntersect<false>(S, ray, tri, t, n, pr);
         if (S.accel == RTB_ACCEL_CONVEX || S.accel == RTB_ACCEL_CONVEX_SIMPLE) return convexIntersect(S, ray, ctx, tri, t, n, pr);
@@ -754,12 +816,12 @@ __device__ bool sceneIntersect(const DScene &S, const Ray &ray, Hit &best, Probe
     });
 }
 // a ray generated by the camera or by a caller carries a fresh context
-template <class Probe>
+template <bool MESH = false, class Probe>
 __device__ bool sceneIntersect(const DScene &S, const Ray &ray, Hit &best, Probe &pr)
 {
     RayCtx ctx;
     ctx.inTunnel = 0; ctx.segment = -1;
-    return sceneIntersect(S, ray, best, pr, ctx);
+    return sceneIntersect<MESH>(S, ray, best, pr, ctx);
 }
 
 // ---------------------------------------------------------------------------------------------

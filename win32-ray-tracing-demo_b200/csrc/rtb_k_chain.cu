@@ -6,7 +6,8 @@ namespace rtb {
 
 template <class Probe, int FOLD> static void go(const Launch &L)
 {
-    k_whitted_chain<Probe, FOLD><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
+    if (L.mesh) k_whitted_chain<Probe, FOLD, true><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
+    else k_whitted_chain<Probe, FOLD><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
 }
 
 void launchChain(const Launch &L)

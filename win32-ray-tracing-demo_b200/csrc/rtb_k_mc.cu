@@ -4,16 +4,18 @@
 
 namespace rtb {
 
-void launchTree(const Launch &L)
+template <bool MESH> static void tree(const Launch &L)
 {
-    if (L.count) k_whitted_tree<CountProbe><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
-    else k_whitted_tree<NoProbe><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
+    if (L.count) k_whitted_tree<CountProbe, MESH><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
+    else k_whitted_tree<NoProbe, MESH><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
 }
+void launchTree(const Launch &L) { if (L.mesh) tree<true>(L); else tree<false>(L); }
 
-void launchMonteCarlo(const Launch &L)
+template <bool MESH> static void monteCarlo(const Launch &L)
 {
-    if (L.count) k_montecarlo<CountProbe><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
-    else k_montecarlo<NoProbe><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
+    if (L.count) k_montecarlo<CountProbe, MESH><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
+    else k_montecarlo<NoProbe, MESH><<<L.grid, RTB_CTA_THREADS, 0, L.stream>>>(*L.S, *L.F, L.out, L.counters);
 }
+void launchMonteCarlo(const Launch &L) { if (L.mesh) monteCarlo<true>(L); else monteCarlo<false>(L); }
 
 } // namespace rtb

@@ -356,12 +356,12 @@ __device__ __forceinline__ V3 chainWith(const DScene &S, const FrameParams &F, i
     return c;
 }
 
-template <int FOLD, class Probe>
+template <int FOLD, bool MESH, class Probe>
 __device__ __forceinline__ V3 chainPerRay(const DScene &S, const FrameParams &F, int x, int y, unsigned int &rays, Probe &pr)
 {
     RayCtx ctx; // carried along the chain: trace() copies it to the reflected ray (MainWindow.cpp:105)
     ctx.inTunnel = 0; ctx.segment = -1;
-    return chainWith<FOLD>(S, F, x, y, rays, pr, [&](const Ray &r, Hit &h) { return sceneIntersect(S, r, h, pr, ctx); });
+    return chainWith<FOLD>(S, F, x, y, rays, pr, [&](const Ray &r, Hit &h) { return sceneIntersect<MESH>(S, r, h, pr, ctx); });
 }
 
 template <class Probe>
@@ -377,7 +377,8 @@ __device__ __forceinline__ void storePixel(const FrameParams &F, float *out, int
     else storeColor(F, out, x, lr, y, c);
 }
 
-template <class Probe, int FOLD>
+// MESH: scenes with RTB_PRIM_MESH records (rtb_device.cuh: sceneIntersectWith)
+template <class Probe, int FOLD, bool MESH = false>
 __global__ void __launch_bounds__(RTB_CTA_THREADS, RTB_CHAIN_MIN_CTAS)
 k_whitted_chain(const __grid_constant__ DScene S, const __grid_constant__ FrameParams F, float *__restrict__ out,
                 Counters *__restrict__ counters)
@@ -391,7 +392,7 @@ k_whitted_chain(const __grid_constant__ DScene S, const __grid_constant__ FrameP
     if (F.skip_heavy && blockIdx.x * (unsigned int)F.warps_per_cta + (threadIdx.x >> 5) < heavyCount(F)) return;
     __shared__ __align__(16) uint32_t stage[RTB_CTA_THREADS / 32][RTB_TILE_STAGE_WORDS];
     V3 c = v3(0, 0, 0);
-    if (active) c = chainPerRay<FOLD>(S, F, x, y, rays, pr);
+    if (active) c = chainPerRay<FOLD, MESH>(S, F, x, y, rays, pr);
     if (!storeGroup(F, out, tile, active, c, stage) && !storeTile(F, out, tile, active, c, stage[threadIdx.x >> 5]) && active)
         storePixel(F, out, x, lr, y, c, t_start, rays, pr);
     finishWarp(F, counters, tile, t_start, rays, ProbeCounts<Probe>::tris(pr), ProbeCounts<Probe>::steps(pr));
@@ -407,7 +408,7 @@ k_whitted_chain(const __grid_constant__ DScene S, const __grid_constant__ FrameP
 #define RTB_TREE_STACK 64 // live items <= 2*max_depth + 1
 struct TreeItem { V3 o, d; float w; int depth; };
 
-template <class Probe>
+template <class Probe, bool MESH = false>
 __global__ void __launch_bounds__(RTB_CTA_THREADS)
 k_whitted_tree(const __grid_constant__ DScene S, const __grid_constant__ FrameParams F, float *__restrict__ out,
                Counters *__restrict__ counters)
@@ -435,7 +436,7 @@ k_whitted_tree(const __grid_constant__ DScene S, const __grid_constant__ FramePa
             int depth = it.depth;
             rays++;
             Hit h;
-            if (!sceneIntersect(S, r, h, pr)) continue;
+            if (!sceneIntersect<MESH>(S, r, h, pr)) continue;
             const rtb_material &m = S.mats[h.mat];
             const V3 nl = (dot(h.n, r.d) < 0) ? h.n : h.n * -1;
             const V3 local = matLocal(m, r, h.pos, h.n);
@@ -484,7 +485,7 @@ struct McItem { V3 o, d, T; int depth; };
 #define RTB_MC_REFERENCE_TRIG 0 // 1: phi = acosf(r2), cosf(phi), sinf(phi), cosf(theta), sinf(theta) literally (MainWindow.cpp:190-197)
 #endif
 
-template <class Probe>
+template <class Probe, bool MESH = false>
 __global__ void __launch_bounds__(RTB_CTA_THREADS, RTB_MC_MIN_CTAS)
 k_montecarlo(const __grid_constant__ DScene S, const __grid_constant__ FrameParams F, float *__restrict__ out,
              Counters *__restrict__ counters)
@@ -538,7 +539,7 @@ k_montecarlo(const __grid_constant__ DScene S, const __grid_constant__ FramePara
             bool alive = false; // does the current path continue with (r, T, depth)?
             rays++;
             Hit h;
-            if (sceneIntersect(S, r, h, pr))
+            if (sceneIntersect<MESH>(S, r, h, pr))
             {
                 const rtb_material &m = smat[h.mat];
                 const V3 n = h.n;

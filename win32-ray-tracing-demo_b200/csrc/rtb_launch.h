@@ -16,6 +16,7 @@ struct Launch
     dim3 grid;           // CTAs of RTB_CTA_THREADS threads
     cudaStream_t stream;
     bool count;          // CountProbe (frame.counters) instead of NoProbe
+    bool mesh;           // the scene has RTB_PRIM_MESH records: the MESH instantiations (chain, tree, Monte Carlo only)
 };
 
 void launchChain(const Launch &L);                // k_whitted_chain        (rtb_k_chain.cu)

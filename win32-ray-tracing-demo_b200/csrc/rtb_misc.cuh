@@ -196,6 +196,7 @@ __global__ void k_kd_relayout(const uint2 *__restrict__ nodes, int n, const unsi
 // ---------------------------------------------------------------------------------------------
 // Parity hooks: primary rays with traversal recording, and arbitrary ray batches
 // ---------------------------------------------------------------------------------------------
+template <bool MESH = false>
 __global__ void __launch_bounds__(RTB_CTA_THREADS)
 k_trace_primary(const __grid_constant__ DScene S, const __grid_constant__ FrameParams F, int *__restrict__ hit_id,
                 float *__restrict__ hit_t, int *__restrict__ seq_len, unsigned long long *__restrict__ seq_hash,
@@ -212,7 +213,7 @@ k_trace_primary(const __grid_constant__ DScene S, const __grid_constant__ FrameP
     pr.buf = seq_buf ? seq_buf + p * seq_cap : nullptr;
     pr.cap = seq_buf ? seq_cap : 0;
     Hit h;
-    const bool ok = sceneIntersect(S, r, h, pr);
+    const bool ok = sceneIntersect<MESH>(S, r, h, pr);
     if (hit_id) hit_id[p] = ok ? h.id : -1;
     if (hit_t) hit_t[p] = ok ? h.t : -1.0f;
     if (seq_len) seq_len[p] = pr.len;
@@ -221,6 +222,7 @@ k_trace_primary(const __grid_constant__ DScene S, const __grid_constant__ FrameP
         for (int i = pr.len; i < seq_cap; i++) seq_buf[p * seq_cap + i] = -1;
 }
 
+template <bool MESH = false>
 __global__ void __launch_bounds__(RTB_CTA_THREADS)
 k_intersect_rays(const __grid_constant__ DScene S, long long n, const float *__restrict__ rays, int *__restrict__ hit_id,
                  float *__restrict__ hit_t, float *__restrict__ position, float *__restrict__ normal)
@@ -232,7 +234,7 @@ k_intersect_rays(const __grid_constant__ DScene S, long long n, const float *__r
     r.d = v3(rays[6 * i + 3], rays[6 * i + 4], rays[6 * i + 5]);
     NoProbe pr;
     Hit h;
-    const bool ok = sceneIntersect(S, r, h, pr);
+    const bool ok = sceneIntersect<MESH>(S, r, h, pr);
     if (hit_id) hit_id[i] = ok ? h.id : -1;
     if (hit_t) hit_t[i] = ok ? h.t : -1.0f;
     if (position) { position[3 * i] = ok ? h.pos.x : 0; position[3 * i + 1] = ok ? h.pos.y : 0; position[3 * i + 2] = ok ? h.pos.z : 0; }
@@ -248,7 +250,7 @@ k_intersect_rays(const __grid_constant__ DScene S, long long n, const float *__r
 // warp-per-pixel render tier: the reference program's own batch is 1000 rays, which as 1000 threads occupies 8 CTAs and
 // takes as long as its longest 200-bounce chain walked by one lane; as 1000 warps it fills the device.  Results are
 // identical (same arithmetic; ties in a list go to the earliest position).  k-d trees and grids only.
-template <bool WIDE>
+template <bool WIDE, bool MESH = false>
 __global__ void __launch_bounds__(RTB_CTA_THREADS)
 k_bounce_rays(const __grid_constant__ DScene S, long long n, const float *__restrict__ rays, int max_depth,
               int *__restrict__ reached, int *__restrict__ depth_out, int *__restrict__ last_id, float *__restrict__ last_pos,
@@ -280,7 +282,7 @@ k_bounce_rays(const __grid_constant__ DScene S, long long n, const float *__rest
                     if (S.accel == RTB_ACCEL_REGULAR_GRID || S.accel == RTB_ACCEL_FLAT_GRID) return gridIntersect<true>(S, r, tri, tt, nn, pr);
                     return kdIntersect<true>(S, r, tri, tt, nn, pr);
                 });
-            else hit = sceneIntersect(S, r, h, pr, ctx);
+            else hit = sceneIntersect<MESH>(S, r, h, pr, ctx);
             if (!hit) { id = -1; break; }
             id = h.id; pos = h.pos;
             const V3 nl = (dot(h.n, r.d) < 0) ? h.n : h.n * -1;

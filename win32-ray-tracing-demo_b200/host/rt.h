@@ -219,6 +219,10 @@ public:
     void setMaterial(const Ptr<Material> &m) { material = m; }
     virtual void flatten(FlatScene &out) const = 0;
     virtual void invalidate();
+    // number of top-level hit ids the geometry takes (GeometrySet::resolveHit): one, a mesh one per triangle
+    virtual int topLevelIds() const { return 1; }
+    // true: topLevelIds() may differ from 1 (and change as the geometry grows)
+    virtual bool variableIds() const { return false; }
 private:
     struct DeviceCache;
     std::shared_ptr<DeviceCache> cache_;
@@ -260,15 +264,35 @@ public:
     void flatten(FlatScene &out) const override;
 };
 
+// A triangle mesh: one RTB_PRIM_MESH record, traversed on the device through a hierarchy built at upload.  It hits what the
+// same triangles added one by one (GeometrySet::addStlFile) hit, with the same ids: triangle k of the mesh is top-level id
+// base + k (include/rtb.h: RTB_PRIM_MESH).  No reference counterpart: the reference loads every facet as a loose Triangle.
+class TriangleMesh : public Geometry
+{
+    std::vector<float> tris; // [n][12]: a, b, c, normal, as the loose_tri records of include/rtb.h
+public:
+    size_t count() const { return tris.size() / 12; }
+    void add(const Point &a, const Point &b, const Point &c, const Vector &normal); // drops the cached device upload
+    void flatten(FlatScene &out) const override;
+    int topLevelIds() const override { return (int)count(); }
+    bool variableIds() const override { return true; }
+protected:
+    Geometry *resolveHit(int id) override;
+};
+
 class GeometrySet : public Geometry
 {
     std::vector<Geometry *> geometries;
+    bool variableIds_ = false; // some geometry may take more or less than one hit id: resolveHit walks the list
 public:
-    void add(Geometry *geometry) { geometries.push_back(geometry); invalidate(); }
+    void add(Geometry *geometry) { geometries.push_back(geometry); variableIds_ = variableIds_ || geometry->variableIds(); invalidate(); }
     Geometry *last() { return geometries.empty() ? nullptr : geometries.back(); }
     size_t size() const { return geometries.size(); }
     bool addStlFile(const char *filename, Ptr<Material> material);
     bool addStlFile(const char *filename, Ptr<Material> material, const Matrix &matrix, const Vector &offset);
+    // the same facets as ONE TriangleMesh (same loose_tri records, same hit ids)
+    bool addStlMesh(const char *filename, Ptr<Material> material);
+    bool addStlMesh(const char *filename, Ptr<Material> material, const Matrix &matrix, const Vector &offset);
     void clear();
     void flatten(FlatScene &out) const override;
     // batch form of intersect(): n rays [n][6] -> results (GPU)
@@ -436,6 +460,7 @@ public:
     int samples;        // valid when FLAG_MONTE_CARLO
     int preset;         // 1..5
     std::string stlPath = "ball.stl";
+    static bool stlAsMeshDefault; // preset 3 loads its STL with addStlMesh instead of addStlFile
     Script(const char *name, int flags, int tunnelSegments, int samples, int preset)
         : name(name), flags(flags), tunnelSegments(tunnelSegments), samples(samples), preset(preset) {}
     virtual ~Script() {}

@@ -182,9 +182,22 @@ struct Geometry::DeviceCache
 void Geometry::invalidate() { cache_.reset(); }
 Geometry *Geometry::resolveHit(int) { return this; }
 
+Geometry *TriangleMesh::resolveHit(int) { return this; }
+
 Geometry *GeometrySet::resolveHit(int id)
 {
-    if (id >= 0 && id < (int)geometries.size()) return geometries[id];
+    if (!variableIds_)
+    { // one id per geometry
+        if (id >= 0 && id < (int)geometries.size()) return geometries[id];
+        return geometries.empty() ? this : geometries.back(); // tunnel triangle ids follow the top-level ones
+    }
+    int base = 0; // a mesh takes one id per triangle
+    for (Geometry *g : geometries)
+    {
+        const int n = g->topLevelIds();
+        if (id >= base && id < base + n) return g;
+        base += n;
+    }
     return geometries.empty() ? this : geometries.back(); // tunnel triangle ids follow the top-level ones
 }
 
@@ -357,8 +370,10 @@ bool Script::Build(GeometrySet &scene, std::unique_ptr<PerspectiveCamera> &camer
             scene.add(mirror);
             scene.add(glass);
         }
-        else if (!scene.addStlFile(stlPath.c_str(), Ptr<Material>(new GlassMaterial()), Matrix(1, 0, 0, 0, 1, 0, 0, 0, 1),
-                                   Vector(50, 0, 40)))
+        else if (stlAsMeshDefault ? !scene.addStlMesh(stlPath.c_str(), Ptr<Material>(new GlassMaterial()), Matrix(1, 0, 0, 0, 1, 0, 0, 0, 1),
+                                                      Vector(50, 0, 40))
+                                  : !scene.addStlFile(stlPath.c_str(), Ptr<Material>(new GlassMaterial()), Matrix(1, 0, 0, 0, 1, 0, 0, 0, 1),
+                                                      Vector(50, 0, 40)))
             return false;
         camera.reset(new PerspectiveCamera(Point(50, 52, 295), Vector(0, -0.045f, -1), Vector(0, 1, -0.045f), 1.3333f, 28, 140.0f));
         setting = RenderSetting::Default();
@@ -401,6 +416,8 @@ void Script::Run(RenderProc render, int tunnelAlgorithm, LogCallback log, Progre
     }
     execTime = render(scene, *camera, setting, progress);
 }
+
+bool Script::stlAsMeshDefault = false;
 
 static Script s1("checker ground and balls", Script::FLAG_MONTE_CARLO, 0, 1000, 1);
 static Script s2("smallpt", Script::FLAG_MONTE_CARLO, 0, 1000, 2);
@@ -478,6 +495,8 @@ void rtbh_set_grid_on_device(int on) { Tunnel::gridOnDeviceDefault = on != 0; }
 void rtbh_set_exact_grid_binning(int on) { Tunnel::exactGridBinningDefault = on != 0; }
 // ... leave their SAH k-d tree to the device builder (Tunnel::kdOnDevice)
 void rtbh_set_kd_on_device(int on) { Tunnel::kdOnDeviceDefault = on != 0; }
+// preset 3 built from now on loads its STL as one mesh (GeometrySet::addStlMesh) instead of loose triangles
+void rtbh_set_stl_as_mesh(int on) { Script::stlAsMeshDefault = on != 0; }
 void rtbh_free(rtbh_scene *h) { delete h; }
 const rtb_flat_scene *rtbh_flat(const rtbh_scene *h) { return &h->flat.view; }
 const rtb_camera *rtbh_camera(const rtbh_scene *h) { return &h->cam; }

@@ -163,12 +163,34 @@ void Triangle::flatten(FlatScene &out) const
     out.prims.push_back(p);
 }
 
+void TriangleMesh::add(const Point &a, const Point &b, const Point &c, const Vector &normal)
+{
+    pushTriangle(tris, a, b, c, normal);
+    invalidate();
+}
+
+void TriangleMesh::flatten(FlatScene &out) const
+{
+    if (tris.empty()) return;
+    rtb_prim p;
+    memset(&p, 0, sizeof(p));
+    p.type = RTB_PRIM_MESH;
+    p.material = out.materialIndex(material.get());
+    p.base_id = out.nTop;
+    p.first = (int)(out.looseTri.size() / 12);
+    p.count = (int)count();
+    out.looseTri.insert(out.looseTri.end(), tris.begin(), tris.end());
+    out.nTop += p.count;
+    out.prims.push_back(p);
+}
+
 GeometrySet::~GeometrySet() { clear(); }
 
 void GeometrySet::clear()
 {
     for (Geometry *g : geometries) delete g;
     geometries.clear();
+    variableIds_ = false;
     invalidate();
 }
 
@@ -177,8 +199,11 @@ bool GeometrySet::addStlFile(const char *filename, Ptr<Material> material)
     return addStlFile(filename, material, Matrix(1, 0, 0, 0, 1, 0, 0, 0, 1), Vector(0, 0, 0));
 }
 
-bool GeometrySet::addStlFile(const char *filename, Ptr<Material> material, const Matrix &matrix, const Vector &offset)
-{ // binary STL: 80-byte header, u32 count, then per facet 12 floats + u16 (reference GeometrySet.cpp:33-86)
+// binary STL: 80-byte header, u32 count, then per facet 12 floats + u16 (reference GeometrySet.cpp:33-86); `facet` receives
+// the transformed vertices and normal of every facet
+template <class Facet>
+static bool readStl(const char *filename, const Matrix &matrix, const Vector &offset, Facet facet)
+{
     FILE *fp = fopen(filename, "rb");
     if (!fp) return false;
     unsigned char header[84];
@@ -197,11 +222,37 @@ bool GeometrySet::addStlFile(const char *filename, Ptr<Material> material, const
         const Point p2 = matrix * Point(f[6], f[7], f[8]) + offset;
         const Point p3 = matrix * Point(f[9], f[10], f[11]) + offset;
         const Vector n = matrix * Vector(f[0], f[1], f[2]).norm();
+        facet(p1, p2, p3, n);
+    }
+    return true;
+}
+
+bool GeometrySet::addStlFile(const char *filename, Ptr<Material> material, const Matrix &matrix, const Vector &offset)
+{
+    const bool ok = readStl(filename, matrix, offset, [&](const Point &p1, const Point &p2, const Point &p3, const Vector &n) {
         Triangle *t = new Triangle(p1, p2, p3, n);
         t->material = material;
         geometries.push_back(t);
+    });
+    if (ok) invalidate();
+    return ok;
+}
+
+bool GeometrySet::addStlMesh(const char *filename, Ptr<Material> material)
+{
+    return addStlMesh(filename, material, Matrix(1, 0, 0, 0, 1, 0, 0, 0, 1), Vector(0, 0, 0));
+}
+
+bool GeometrySet::addStlMesh(const char *filename, Ptr<Material> material, const Matrix &matrix, const Vector &offset)
+{
+    TriangleMesh *mesh = new TriangleMesh();
+    mesh->material = material;
+    if (!readStl(filename, matrix, offset, [&](const Point &p1, const Point &p2, const Point &p3, const Vector &n) { mesh->add(p1, p2, p3, n); }))
+    {
+        delete mesh;
+        return false;
     }
-    invalidate();
+    add(mesh);
     return true;
 }
 
