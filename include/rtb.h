@@ -291,6 +291,25 @@ typedef struct rtb_bvhnode {
 int rtb_scene_mesh_download(rtb_ctx *ctx, const rtb_scene *scene, int32_t mesh_index, rtb_bvhnode *nodes, int64_t node_cap,
                             uint32_t *tri_order, int64_t tri_cap, int64_t counts[3]);
 
+/* Replace the triangles of the MESH record `mesh_index` (0 = first MESH record in prims order): `tri` = [n][12] records in
+ * the loose_tri format (a, b, c, normal), n == the record's count.  `tri` is host memory (pageable or page-locked; staged,
+ * reusable when the call returns) or device memory of the context's device (16-byte aligned; read in place, no PCIe);
+ * managed memory is read in place on the device like device memory.
+ * Enqueued behind the work already on `stream` (0 = the context's stream, which is not ordered with the legacy default
+ * stream: pass cudaStreamLegacy for that) and behind every launch that reads the scene;
+ * later work on `stream` and later renders on any stream see the new triangles.  No host synchronisation for a device source.
+ * The scene becomes the one rtb_scene_upload gives for the same flat scene with loose_tri[first, first + count) replaced:
+ * TRIANGLES runs over that range see the new records, and every other MESH record that intersects the range must lie inside
+ * it (its records are a slice of `tri`; it gets the same operation) -- one that overlaps it only in part is
+ * RTB_ERR_UNSUPPORTED.  Every rejection leaves the scene unchanged: n != count and device memory of another device or
+ * misaligned are RTB_ERR_INVALID, no such mesh is RTB_ERR_UNSUPPORTED.
+ *   RTB_MESH_REBUILD: the hierarchy is built again as rtb_scene_upload builds it (byte-identical tree, identical results).
+ *   RTB_MESH_REFIT:   child links and leaf order are kept, every box is recomputed from the new records (the bound of the
+ *                     node test holds for any tree shape: the mesh contract holds; the tree's quality decays with large motion). */
+enum { RTB_MESH_REBUILD = 0, RTB_MESH_REFIT = 1 };
+int rtb_scene_mesh_update(rtb_ctx *ctx, rtb_scene *scene, int32_t mesh_index, const float *tri, int64_t n,
+                          int32_t flags, void *stream);
+
 /* Replaces `int Render(GeometrySet&, PerspectiveCamera&, RenderSetting&, ProgressCallback)`
  * (reference MainWindow.cpp:251-303, the RenderProc of Scripts.h:11-12): ray generation,
  * trace()/radiance() and the framebuffer store for this rank's rows.  `rgb_out` is a HOST
@@ -404,6 +423,9 @@ int rtb_multi_scene_free(rtb_multi *m, rtb_multi_scene *scene);
 int64_t rtb_multi_scene_upload_bytes(const rtb_multi_scene *scene); /* summed over the devices */
 int rtb_multi_render(rtb_multi *m, const rtb_multi_scene *scene, const rtb_camera *camera,
                      const rtb_render_setting *setting, const rtb_frame *frame, void *rgb_out, rtb_stats *stats);
+/* rtb_scene_mesh_update on every device of the scene; `tri` is host memory (device and managed memory are RTB_ERR_INVALID). */
+int rtb_multi_scene_mesh_update(rtb_multi *m, rtb_multi_scene *scene, int32_t mesh_index, const float *tri, int64_t n,
+                                int32_t flags);
 
 #ifdef __cplusplus
 }

@@ -23,6 +23,8 @@ STAT_NAMES = ["n_top", "n_tris", "grid_x", "grid_y", "grid_z", "cells_nonempty",
 LAYOUT_ROWMAJOR, LAYOUT_REFERENCE, LAYOUT_GLOBAL, OUTPUT_RGB8, OUTPUT_MOMENTS = 0, 1, 2, 4, 8
 IPC_HANDLE_BYTES = 64
 PRIM_PLANE, PRIM_SPHERE, PRIM_TRIANGLES, PRIM_TUNNEL, PRIM_MESH = 0, 1, 2, 3, 4  # rtb_prim.type
+MESH_REBUILD, MESH_REFIT = 0, 1  # rtb_scene_mesh_update flags
+CUDA_STREAM_LEGACY = 1  # cudaStreamLegacy
 
 
 class RtbError(RuntimeError):
@@ -132,12 +134,13 @@ class Stats(C.Structure):
 ABI_SYMBOLS = ["rtb_init", "rtb_shutdown", "rtb_last_error", "rtb_abi_version", "rtb_shard_rows", "rtb_shard_width",
                "rtb_unshard_cols_device",
                "rtb_host_alloc", "rtb_host_free", "rtb_host_register", "rtb_host_unregister",
-               "rtb_scene_upload", "rtb_scene_free", "rtb_scene_device_bytes", "rtb_scene_upload_bytes", "rtb_scene_grid_hash", "rtb_scene_kd_download", "rtb_scene_mesh_download", "rtb_render",
+               "rtb_scene_upload", "rtb_scene_free", "rtb_scene_device_bytes", "rtb_scene_upload_bytes", "rtb_scene_grid_hash", "rtb_scene_kd_download", "rtb_scene_mesh_download", "rtb_scene_mesh_update", "rtb_render",
                "rtb_render_device", "rtb_unshard_device", "rtb_trace_primary", "rtb_intersect_rays", "rtb_bounce_rays",
                "rtb_selftest_pretest", "rtb_kd_validate", "rtb_forget_schedule", "rtb_set_progress", "rtb_multi_set_progress",
                "rtb_device_alloc", "rtb_device_free", "rtb_device_download", "rtb_ipc_export", "rtb_ipc_open", "rtb_ipc_close", "rtb_scatter_shard_device",
                "rtb_multi_init", "rtb_multi_shutdown", "rtb_multi_count", "rtb_multi_ctx", "rtb_multi_last_error",
-               "rtb_multi_scene_upload", "rtb_multi_scene_free", "rtb_multi_scene_upload_bytes", "rtb_multi_render"]
+               "rtb_multi_scene_upload", "rtb_multi_scene_free", "rtb_multi_scene_upload_bytes", "rtb_multi_render",
+               "rtb_multi_scene_mesh_update"]
 
 _cuda = None
 _host = None
@@ -173,6 +176,7 @@ def cuda_lib():
         lib.rtb_scene_grid_hash.restype = C.c_int
         lib.rtb_scene_kd_download.argtypes = [vp, vp, vp, i64, vp, i64, C.POINTER(C.c_int64), C.POINTER(C.c_float)]
         lib.rtb_scene_mesh_download.argtypes = [vp, vp, i32, vp, i64, vp, i64, C.POINTER(C.c_int64)]
+        lib.rtb_scene_mesh_update.argtypes = [vp, vp, i32, vp, i64, i32, vp]
         lib.rtb_render.argtypes = [vp, vp, C.POINTER(Camera), C.POINTER(RenderSetting), C.POINTER(Frame), vp,
                                    C.POINTER(Stats)]
         lib.rtb_render_device.argtypes = [vp, vp, C.POINTER(Camera), C.POINTER(RenderSetting), C.POINTER(Frame),
@@ -201,6 +205,7 @@ def cuda_lib():
         lib.rtb_multi_scene_upload_bytes.argtypes = [vp]
         lib.rtb_multi_scene_upload_bytes.restype = i64
         lib.rtb_multi_render.argtypes = [vp, vp, C.POINTER(Camera), C.POINTER(RenderSetting), C.POINTER(Frame), vp, C.POINTER(Stats)]
+        lib.rtb_multi_scene_mesh_update.argtypes = [vp, vp, i32, vp, i64, i32]
         _cuda = lib
     return _cuda
 
@@ -556,6 +561,12 @@ class MultiScene:
     def upload_bytes(self):
         return int(self.multi._lib.rtb_multi_scene_upload_bytes(self._h))
 
+    def mesh_update(self, records, mesh_index=0, refit=False):
+        """rtb_multi_scene_mesh_update: DeviceScene.mesh_update on every device; `records` is a [count][12] float32 numpy array."""
+        rec = _host_records(records)
+        self.multi._check(self.multi._lib.rtb_multi_scene_mesh_update(self.multi._h, self._h, mesh_index, rec.ctypes.data, len(rec),
+                                                                      MESH_REFIT if refit else MESH_REBUILD), "rtb_multi_scene_mesh_update")
+
     def render(self, camera, setting, frame, out=None):
         """The whole frame into ONE host buffer: [height][width][3] (reference order [width][height][3] with LAYOUT_REFERENCE)."""
         if out is None:
@@ -577,6 +588,10 @@ def unshard_device(ctx, gathered_ptr, image_ptr, width, height, world, row_block
 def unshard_cols_device(ctx, gathered_ptr, image_ptr, width, height, world, row_block, col_block, stream=0):
     ctx._check(ctx._lib.rtb_unshard_cols_device(ctx._h, C.c_void_p(gathered_ptr), C.c_void_p(image_ptr), width, height, world,
                                                 row_block, col_block, C.c_void_p(stream)), "rtb_unshard_cols_device")
+
+
+def _host_records(records):
+    return np.ascontiguousarray(records, np.float32).reshape(-1, 12)
 
 
 class PinnedArray:
@@ -703,6 +718,29 @@ class DeviceScene:
         f = raw[:, :48].copy().view(np.float32).reshape(-1, 12)
         child = raw[:, 48:56].copy().view(np.int32).reshape(-1, 2)
         return f[:, :6].reshape(-1, 2, 3), f[:, 6:].reshape(-1, 2, 3), child, order, int(counts[2])
+
+    def mesh_update(self, records, mesh_index=0, refit=False, stream=None):
+        """rtb_scene_mesh_update: replace the triangles of the mesh record `mesh_index` (include/rtb.h).  `records` is a
+        [count][12] float32 numpy array (a, b, c, normal: the loose_tri format), or a contiguous CUDA float32 tensor on the
+        context's device, read in place behind the work on `stream` (default: torch's current stream, its default stream
+        included; an explicit 0 is the context's own stream).  refit=False
+        rebuilds the hierarchy as an upload does; refit=True keeps its shape and recomputes its boxes."""
+        flags = MESH_REFIT if refit else MESH_REBUILD
+        if hasattr(records, "data_ptr"):  # a torch tensor
+            import torch
+            if not records.is_cuda or records.dtype != torch.float32 or not records.is_contiguous() or records.numel() % 12:
+                raise RtbError("mesh_update: a tensor must be a contiguous CUDA float32 tensor of [count][12] records")
+            if stream is None:
+                stream = torch.cuda.current_stream(records.device).cuda_stream
+                # torch's default stream has handle 0, which the library reads as its own stream (not ordered with the
+                # legacy default stream): name the legacy stream instead
+                stream = stream or CUDA_STREAM_LEGACY
+            ptr, n = records.data_ptr(), records.numel() // 12
+        else:
+            rec = _host_records(records)
+            ptr, n = rec.ctypes.data, len(rec)
+        self.ctx._check(self.ctx._lib.rtb_scene_mesh_update(self.ctx._h, self._h, mesh_index, C.c_void_p(ptr), n, flags,
+                                                            C.c_void_p(stream or 0)), "rtb_scene_mesh_update")
 
     def render(self, camera, setting, frame, out=None):
         """rtb_render with HOST buffers; returns (rows x width x 3 float32 | reference-order array, stats)."""

@@ -224,6 +224,7 @@ struct rtb_ctx
     cudaStream_t aux = nullptr;                 // high-priority side stream of the latency-critical tiles
     cudaEvent_t fork = nullptr, join = nullptr;
     cudaEvent_t last_frame = nullptr;      // recorded behind the last kernel of every frame (waitLastFrame)
+    cudaEvent_t caller_ready = nullptr;    // rtb_scene_mesh_update: the caller's stream, awaited by ctx->stream
     cudaStream_t last_frame_stream = nullptr;
     bool frame_pending = false;
     float *d_frame = nullptr; // grow-only device framebuffer of the host-buffer render call
@@ -389,6 +390,7 @@ extern "C" int rtb_shutdown(rtb_ctx *ctx)
     if (ctx->frame_pending) cudaEventSynchronize(ctx->last_frame); // a frame on a caller's stream
     cudaStreamSynchronize(ctx->stream);
     if (ctx->last_frame) cudaEventDestroy(ctx->last_frame);
+    if (ctx->caller_ready) cudaEventDestroy(ctx->caller_ready);
     for (int i = 0; i < 4; i++)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     if (ctx->aux) { cudaStreamSynchronize(ctx->aux); cudaStreamDestroy(ctx->aux); }
@@ -1161,6 +1163,67 @@ static size_t stagedBytesBound(const rtb_flat_scene *f)
     return t + 4096;
 }
 
+// Temporaries of the per-record hierarchy builds and refits, sized for the largest record; released stream-ordered.
+struct MeshScratch
+{
+    cudaStream_t st = nullptr;
+    size_t maxN = 0, tmpBytes = 0;
+    unsigned int *bounds = nullptr, *arrivals = nullptr;
+    unsigned long long *keys = nullptr, *sorted = nullptr;
+    int *parent = nullptr; // inner nodes' links at [0, maxN), leaves' at [maxN, 2 maxN)
+    void *tmp = nullptr;
+    std::vector<void *> temps;
+    // rebuild = false: only what a refit uses (arrivals and parent links)
+    cudaError_t alloc(cudaStream_t stream, size_t n, bool rebuild)
+    {
+        st = stream;
+        maxN = n;
+        auto temp = [&](size_t bytes, void **p) { cudaError_t e = cudaMallocAsync(p, bytes ? bytes : 1, st); if (e == cudaSuccess) temps.push_back(*p); return e; };
+        cudaError_t e;
+        if ((e = temp(maxN * sizeof(unsigned int), (void **)&arrivals)) != cudaSuccess) return e;
+        if ((e = temp(2 * maxN * sizeof(int), (void **)&parent)) != cudaSuccess) return e;
+        if (!rebuild) return cudaSuccess;
+        if ((e = cub::DeviceRadixSort::SortKeys(nullptr, tmpBytes, keys, sorted, (int)maxN, 0, 62, st)) != cudaSuccess) return e;
+        if ((e = temp(6 * sizeof(unsigned int), (void **)&bounds)) != cudaSuccess) return e;
+        if ((e = temp(maxN * sizeof(unsigned long long), (void **)&keys)) != cudaSuccess) return e;
+        if ((e = temp(maxN * sizeof(unsigned long long), (void **)&sorted)) != cudaSuccess) return e;
+        return temp(tmpBytes, &tmp);
+    }
+    ~MeshScratch() { for (void *p : temps) cudaFreeAsync(p, st); }
+};
+
+// The hierarchy of MESH record i from its raw records `raw` ([count][12] on the device) and its packed records, already in
+// DScene::loose.  rebuild: the whole LBVH pipeline (what rtb_scene_upload runs); otherwise a refit: child links and leaf
+// order are kept, every box is computed again from the new records.
+static int meshRecord(rtb_ctx *ctx, rtb_scene *s, int i, const float *raw, MeshScratch &t, bool rebuild)
+{
+    DScene &d = s->d;
+    const cudaStream_t st = t.st;
+    const rtb_prim &P = d.prims[i];
+    const int n = P.count;
+    const unsigned int tb = 256, nb = (unsigned int)((n + tb - 1) / tb), nbInner = (unsigned int)((n - 1 + tb - 1) / tb);
+    const size_t base = (size_t)d.mesh_base[i];
+    rtb_bvhnode *nodes = reinterpret_cast<rtb_bvhnode *>(const_cast<float4 *>(d.mesh_nodes)) + base;
+    uint32_t *order = const_cast<uint32_t *>(d.mesh_order) + base;
+    if (rebuild)
+    {
+        CUDA_TRY(ctx, cudaMemsetAsync(t.bounds, 0xff, 3 * sizeof(unsigned int), st));
+        CUDA_TRY(ctx, cudaMemsetAsync(t.bounds + 3, 0, 3 * sizeof(unsigned int), st));
+        k_bvh_bounds<<<nb, tb, 0, st>>>(raw, n, t.bounds);
+        k_bvh_keys<<<nb, tb, 0, st>>>(raw, n, t.bounds, t.keys);
+        size_t need = t.tmpBytes;
+        CUDA_TRY(ctx, cub::DeviceRadixSort::SortKeys(t.tmp, need, t.keys, t.sorted, n, 0, 62, st));
+        if (n > 1) k_bvh_hierarchy<<<nbInner, tb, 0, st>>>(t.sorted, n, nodes, t.parent, t.parent + t.maxN);
+        k_bvh_order<<<nb, tb, 0, st>>>(t.sorted, n, order);
+    }
+    else if (n > 1) k_bvh_parents<<<nbInner, tb, 0, st>>>(nodes, n, t.parent, t.parent + t.maxN);
+    CUDA_TRY(ctx, cudaMemsetAsync(t.arrivals, 0, (size_t)n * sizeof(unsigned int), st));
+    k_bvh_boxes<<<nb, tb, 0, st>>>(raw, order, n, nodes, t.parent, t.parent + t.maxN, t.arrivals);
+    k_bvh_leaves<<<nb, tb, 0, st>>>(d.loose + 3ull * (unsigned int)P.first, order, n, const_cast<float4 *>(d.mesh_tris) + 3 * base);
+    CUDA_TRY(ctx, cudaGetLastError());
+    return RTB_OK;
+}
+
 // Hierarchies of the MESH records (rtb_build_bvh.cuh) from the raw loose records on the device.  Every record gets its own
 // slice of the three arrays (DScene::mesh_base: the mesh triangles of the records before it), so records whose loose ranges
 // overlap each have their own tree; a mesh of n triangles uses max(n - 1, 1) <= n node slots (the spare one stays zero).
@@ -1169,11 +1232,12 @@ static int buildMeshesOnDevice(rtb_ctx *ctx, rtb_scene *s, const float *d_raw)
     DScene &d = s->d;
     cudaStream_t st = ctx->stream;
     int rc;
-    size_t total = 0;
+    size_t total = 0, maxN = 0;
     for (int i : s->mesh_prims)
     {
         d.mesh_base[i] = (int)total;
         total += (size_t)d.prims[i].count;
+        maxN = std::max(maxN, (size_t)d.prims[i].count);
     }
     if (total > 0x7fffffffull) return fail(ctx, RTB_ERR_UNSUPPORTED, "rtb_scene_upload: more than 2^31 - 1 mesh triangles in all");
     rtb_bvhnode *nodes = nullptr;
@@ -1186,46 +1250,10 @@ static int buildMeshesOnDevice(rtb_ctx *ctx, rtb_scene *s, const float *d_raw)
     d.mesh_nodes = reinterpret_cast<const float4 *>(nodes);
     d.mesh_tris = tris;
     d.mesh_order = order;
-    std::vector<void *> temps;
-    auto temp = [&](size_t bytes, void **p) { cudaError_t e = cudaMallocAsync(p, bytes ? bytes : 1, st); if (e == cudaSuccess) temps.push_back(*p); return e; };
-    auto cleanup = [&]() { for (void *p : temps) cudaFreeAsync(p, st); };
-#define MESH_TRY(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { cleanup(); return fail(ctx, RTB_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } } while (0)
-    size_t maxN = 0;
-    for (int i : s->mesh_prims) maxN = std::max(maxN, (size_t)d.prims[i].count);
-    unsigned int *d_bounds = nullptr, *d_arrivals = nullptr;
-    unsigned long long *d_keys = nullptr, *d_sorted = nullptr;
-    int *d_parent = nullptr;
-    void *d_tmp = nullptr;
-    size_t tmpBytes = 0;
-    MESH_TRY(cub::DeviceRadixSort::SortKeys(nullptr, tmpBytes, d_keys, d_sorted, (int)maxN, 0, 62, st));
-    MESH_TRY(temp(6 * sizeof(unsigned int), (void **)&d_bounds));
-    MESH_TRY(temp(maxN * sizeof(unsigned int), (void **)&d_arrivals));
-    MESH_TRY(temp(maxN * sizeof(unsigned long long), (void **)&d_keys));
-    MESH_TRY(temp(maxN * sizeof(unsigned long long), (void **)&d_sorted));
-    MESH_TRY(temp(2 * maxN * sizeof(int), (void **)&d_parent));
-    MESH_TRY(temp(tmpBytes, &d_tmp));
+    MeshScratch t;
+    CUDA_TRY(ctx, t.alloc(st, maxN, true));
     for (int i : s->mesh_prims)
-    {
-        const rtb_prim &P = d.prims[i];
-        const int n = P.count;
-        const unsigned int tb = 256, nb = (unsigned int)((n + tb - 1) / tb);
-        const float *raw = d_raw + 12ull * (unsigned int)P.first;
-        MESH_TRY(cudaMemsetAsync(d_bounds, 0xff, 3 * sizeof(unsigned int), st));
-        MESH_TRY(cudaMemsetAsync(d_bounds + 3, 0, 3 * sizeof(unsigned int), st));
-        MESH_TRY(cudaMemsetAsync(d_arrivals, 0, (size_t)n * sizeof(unsigned int), st));
-        k_bvh_bounds<<<nb, tb, 0, st>>>(raw, n, d_bounds);
-        k_bvh_keys<<<nb, tb, 0, st>>>(raw, n, d_bounds, d_keys);
-        size_t need = tmpBytes;
-        MESH_TRY(cub::DeviceRadixSort::SortKeys(d_tmp, need, d_keys, d_sorted, n, 0, 62, st));
-        const size_t base = (size_t)d.mesh_base[i];
-        rtb_bvhnode *mn = nodes + base;
-        if (n > 1) k_bvh_hierarchy<<<(unsigned int)((n - 1 + tb - 1) / tb), tb, 0, st>>>(d_sorted, n, mn, d_parent, d_parent + maxN);
-        k_bvh_boxes<<<nb, tb, 0, st>>>(raw, d_sorted, n, mn, d_parent, d_parent + maxN, d_arrivals);
-        k_bvh_leaves<<<nb, tb, 0, st>>>(d.loose + 3ull * (unsigned int)P.first, d_sorted, n, tris + 3 * base, order + base);
-        MESH_TRY(cudaGetLastError());
-    }
-#undef MESH_TRY
-    cleanup();
+        if ((rc = meshRecord(ctx, s, i, d_raw + 12ull * (unsigned int)d.prims[i].first, t, true)) != RTB_OK) return rc;
     return RTB_OK;
 }
 
@@ -1563,6 +1591,103 @@ extern "C" int rtb_scene_mesh_download(rtb_ctx *ctx, const rtb_scene *s, int32_t
         counts[0] = nNodes; counts[1] = P.count; counts[2] = depth;
     }
     return RTB_OK;
+}
+
+// ---- mesh update ------------------------------------------------------------------------------
+// The MESH records an update of record `mesh_index` with n records rewrites: that record, then every other MESH record whose
+// range intersects its range (which must lie inside it).  Every check of the update is here, before anything is written.
+static int meshUpdateRecords(rtb_ctx *ctx, const rtb_scene *s, int32_t mesh_index, int64_t n, int32_t flags, std::vector<int> &recs)
+{
+    if (flags != RTB_MESH_REBUILD && flags != RTB_MESH_REFIT) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_update: unknown flags");
+    if (mesh_index < 0 || mesh_index >= (int32_t)s->mesh_prims.size())
+        return fail(ctx, RTB_ERR_UNSUPPORTED, "rtb_scene_mesh_update: the scene has no such mesh record");
+    const int target = s->mesh_prims[(size_t)mesh_index];
+    const rtb_prim &M = s->d.prims[target];
+    if (n != M.count) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_update: n differs from the mesh record's count");
+    const int64_t first = M.first, end = (int64_t)M.first + M.count;
+    recs.assign(1, target);
+    for (int j : s->mesh_prims)
+    {
+        const rtb_prim &P = s->d.prims[j];
+        const int64_t b = P.first, e = (int64_t)P.first + P.count;
+        if (j == target || e <= first || b >= end) continue;
+        if (b < first || e > end)
+            return fail(ctx, RTB_ERR_UNSUPPORTED, "rtb_scene_mesh_update: mesh record " + std::to_string(j) +
+                                                      " overlaps the updated range only in part");
+        recs.push_back(j);
+    }
+    return RTB_OK;
+}
+
+// Enqueue the update on ctx->stream behind `caller` and every launch that has read the scene; `caller` waits for it.  `src`
+// holds the records of the whole range: device memory of this device, or page-locked host memory (staged) when `host`.
+static int meshUpdateEnqueue(rtb_ctx *ctx, rtb_scene *s, const std::vector<int> &recs, const float *src, bool host, int32_t flags,
+                             cudaStream_t caller)
+{
+    DScene &d = s->d;
+    const cudaStream_t st = ctx->stream;
+    const rtb_prim &M = d.prims[recs[0]];
+    const size_t n = (size_t)M.count, bytes = n * 12 * sizeof(float);
+    if (caller != st)
+    {
+        if (!ctx->caller_ready) CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->caller_ready, cudaEventDisableTiming));
+        CUDA_TRY(ctx, cudaEventRecord(ctx->caller_ready, caller));
+        CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->caller_ready, 0));
+    }
+    // renders on other streams record last_use behind their kernels, and frames of a context run one after the other
+    // (waitLastFrame): the last one covers them all
+    CUDA_TRY(ctx, cudaStreamWaitEvent(st, s->last_use, 0));
+    // every allocation comes before the first write to the scene: a failed one leaves the scene as it was
+    struct RawGuard { void *p = nullptr; cudaStream_t st; ~RawGuard() { if (p) cudaFreeAsync(p, st); } } raw{nullptr, st};
+    MeshScratch t;
+    if (host) CUDA_TRY(ctx, cudaMallocAsync(&raw.p, bytes, st));
+    CUDA_TRY(ctx, t.alloc(st, n, flags == RTB_MESH_REBUILD));
+    if (host)
+    {
+        CUDA_TRY(ctx, cudaMemcpyAsync(raw.p, src, bytes, cudaMemcpyHostToDevice, st));
+        src = (const float *)raw.p;
+    }
+    k_pack_triangles<<<(unsigned int)((n + 255) / 256), 256, 0, st>>>(src, (int)n, const_cast<float4 *>(d.loose) + 3ull * (unsigned int)M.first, nullptr);
+    CUDA_TRY(ctx, cudaGetLastError());
+    for (int i : recs)
+    {
+        const int rc = meshRecord(ctx, s, i, src + 12ull * (unsigned int)(d.prims[i].first - M.first), t, flags == RTB_MESH_REBUILD);
+        if (rc != RTB_OK) return rc;
+    }
+    CUDA_TRY(ctx, cudaEventRecord(s->ready, st));
+    if (caller != st) CUDA_TRY(ctx, cudaStreamWaitEvent(caller, s->ready, 0));
+    return RTB_OK;
+}
+
+extern "C" int rtb_scene_mesh_update(rtb_ctx *ctx, rtb_scene *s, int32_t mesh_index, const float *tri, int64_t n, int32_t flags,
+                                     void *stream)
+{
+    if (!ctx || !s || !tri) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_update: null argument");
+    std::vector<int> recs;
+    int rc = meshUpdateRecords(ctx, s, mesh_index, n, flags, recs);
+    if (rc != RTB_OK) return rc;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    cudaPointerAttributes attr;
+    const bool known = cudaPointerGetAttributes(&attr, tri) == cudaSuccess;
+    cudaGetLastError();
+    // managed memory may still be written by work on `stream`: it is read on the device, in stream order, like device memory
+    const bool managed = known && attr.type == cudaMemoryTypeManaged;
+    const bool onDevice = managed || (known && attr.type == cudaMemoryTypeDevice);
+    const float *src = tri;
+    if (onDevice)
+    {
+        if (!managed && attr.device != ctx->device) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_update: the records are on another device");
+        if ((uintptr_t)tri & 15u) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_update: device records must be 16-byte aligned");
+    }
+    else
+    { // staged: the caller may reuse its array when the call returns
+        char *staged = nullptr;
+        const size_t bytes = (size_t)n * 12 * sizeof(float);
+        if ((rc = stageReserve(ctx, bytes, &staged)) != RTB_OK) return rc;
+        memcpy(staged, tri, bytes);
+        src = (const float *)staged;
+    }
+    return meshUpdateEnqueue(ctx, s, recs, src, !onDevice, flags, stream ? (cudaStream_t)stream : ctx->stream);
 }
 
 // ---- render -----------------------------------------------------------------------------------
@@ -2227,6 +2352,35 @@ extern "C" int rtb_multi_scene_upload(rtb_multi *m, const rtb_flat_scene *flat, 
             return failMulti(m, code, msg);
         }
     *out = s;
+    return RTB_OK;
+}
+
+extern "C" int rtb_multi_scene_mesh_update(rtb_multi *m, rtb_multi_scene *s, int32_t mesh_index, const float *tri, int64_t n,
+                                           int32_t flags)
+{
+    if (!m || !s || !tri || s->s.size() != m->ctx.size()) return failMulti(m, RTB_ERR_INVALID, "rtb_multi_scene_mesh_update: null argument");
+    rtb_ctx *c0 = m->ctx[0];
+    std::vector<int> recs; // every device holds the same records: the checks on the first one hold for all
+    int rc = meshUpdateRecords(c0, s->s[0], mesh_index, n, flags, recs);
+    if (rc != RTB_OK) return failMulti(m, rc, c0->error);
+    if (cudaSetDevice(c0->device) != cudaSuccess) return failMulti(m, RTB_ERR_CUDA, "rtb_multi_scene_mesh_update: cudaSetDevice failed");
+    cudaPointerAttributes attr;
+    const bool onDevice = cudaPointerGetAttributes(&attr, tri) == cudaSuccess &&
+                          (attr.type == cudaMemoryTypeDevice || attr.type == cudaMemoryTypeManaged);
+    cudaGetLastError();
+    if (onDevice) return failMulti(m, RTB_ERR_INVALID, "rtb_multi_scene_mesh_update: the records must be host memory (not device or managed)");
+    // staged once, in the first context's ring: every device copies from it (the ring is reused only after they all drained)
+    const size_t bytes = (size_t)n * 12 * sizeof(float);
+    char *staged = nullptr;
+    if ((rc = stageReserve(c0, bytes, &staged)) != RTB_OK) return failMulti(m, rc, c0->error);
+    memcpy(staged, tri, bytes);
+    for (size_t i = 0; i < m->ctx.size(); i++)
+    {
+        rtb_ctx *c = m->ctx[i];
+        if (cudaSetDevice(c->device) != cudaSuccess) return failMulti(m, RTB_ERR_CUDA, "rtb_multi_scene_mesh_update: cudaSetDevice failed");
+        if ((rc = meshUpdateEnqueue(c, s->s[i], recs, (const float *)staged, true, flags, c->stream)) != RTB_OK)
+            return failMulti(m, rc, "device " + std::to_string(c->device) + ": " + c->error);
+    }
     return RTB_OK;
 }
 

@@ -6,9 +6,12 @@
 //      inner node splits on a strictly lower bit than its parent and the depth of inner nodes is at most 62;
 //   3. radix sort of the keys;
 //   4. hierarchy: inner node i covers a key range found from the common-prefix lengths of its neighbours;
-//   5. boxes bottom-up: the second thread to reach a node takes the union of its two child boxes (float min / max only);
-//   6. the triangle records (exact stream) copied into leaf order, with the local index of each leaf.
+//   5. the local index of each leaf (the leaf order);
+//   6. boxes bottom-up: the second thread to reach a node takes the union of its two child boxes (float min / max only);
+//   7. the triangle records (exact stream) copied into leaf order.
 // Every step is a deterministic function of the input: two builds of the same mesh are byte-identical.
+// A refit (rtb_scene_mesh_update) keeps the child links and the leaf order: it derives the parent links from the child links
+// (k_bvh_parents) and runs steps 6 and 7 again on the new records.
 #pragma once
 #include <cub/cub.cuh>
 #include "rtb_bvh.h"
@@ -108,15 +111,34 @@ __global__ void k_bvh_hierarchy(const unsigned long long *__restrict__ keys, int
     if (right < 0) parent_leaf[~right] = 2 * i + 1; else parent_inner[right] = 2 * i + 1;
 }
 
+// the parent links of a built hierarchy (the layout k_bvh_hierarchy writes), from its child links: inner node i of n - 1
+__global__ void k_bvh_parents(const rtb_bvhnode *__restrict__ nodes, int n, int *__restrict__ parent_inner, int *__restrict__ parent_leaf)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n - 1) return;
+    for (int side = 0; side < 2; side++)
+    {
+        const int c = nodes[i].child[side];
+        if (c < 0) parent_leaf[~c] = 2 * i + side; else parent_inner[c] = 2 * i + side;
+    }
+}
+
+// the local index of the triangle at each leaf position: the low half of its sorted key
+__global__ void k_bvh_order(const unsigned long long *__restrict__ keys, int n, uint32_t *__restrict__ leaf_order)
+{
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p < n) leaf_order[p] = (uint32_t)(keys[p] & 0xffffffffull);
+}
+
 // one thread per leaf position p: leaf box into its parent's slot, then up while this thread is the second to arrive
-__global__ void k_bvh_boxes(const float *__restrict__ raw, const unsigned long long *__restrict__ keys, int n,
+__global__ void k_bvh_boxes(const float *__restrict__ raw, const uint32_t *__restrict__ leaf_order, int n,
                             rtb_bvhnode *__restrict__ nodes, const int *__restrict__ parent_inner,
                             const int *__restrict__ parent_leaf, unsigned int *__restrict__ arrivals)
 {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n) return;
     float lo[3], hi[3];
-    rtb_bvh::leafBox(raw + 12ull * (unsigned int)(keys[p] & 0xffffffffull), lo, hi);
+    rtb_bvh::leafBox(raw + 12ull * leaf_order[p], lo, hi);
     if (n == 1)
     { // a single leaf: both links of the root point at it
         for (int c = 0; c < 2; c++)
@@ -146,15 +168,14 @@ __global__ void k_bvh_boxes(const float *__restrict__ raw, const unsigned long l
     }
 }
 
-// triangle records in leaf order, and the local index of each leaf
-__global__ void k_bvh_leaves(const float4 *__restrict__ exact, const unsigned long long *__restrict__ keys, int n,
-                             float4 *__restrict__ leaf_tris, uint32_t *__restrict__ leaf_order)
+// triangle records in leaf order
+__global__ void k_bvh_leaves(const float4 *__restrict__ exact, const uint32_t *__restrict__ leaf_order, int n,
+                             float4 *__restrict__ leaf_tris)
 {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n) return;
-    const unsigned int k = (unsigned int)(keys[p] & 0xffffffffull);
+    const unsigned int k = leaf_order[p];
     for (int j = 0; j < 3; j++) leaf_tris[3ull * p + j] = exact[3ull * k + j];
-    leaf_order[p] = k;
 }
 
 } // namespace rtb
