@@ -349,6 +349,29 @@ int rtb_trace_primary(rtb_ctx *ctx, const rtb_scene *scene, const rtb_camera *ca
 int rtb_intersect_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *rays,
                        int32_t *hit_id, float *hit_t, float *position, float *normal);
 
+/* Ray queries on DEVICE buffers, stream-ordered (no host synchronisation, no allocation): for a physics or robotics step,
+ * a sensor model or a renderer outside this library that keep their rays on the device.
+ * rays = [n][6] origin, direction: memory of the context's device or managed memory, 8-byte aligned.  tmax = [n] per-ray
+ * bounds in the same kind of memory, or NULL: tmax_all for every ray.  Every other buffer is such memory too.
+ *   RTB_QUERY_CLOSEST: hit_id, hit_t, position, normal (any may be NULL; occluded must be NULL) as rtb_intersect_rays
+ *     writes them.  The bound is STRICT: a ray's result is rtb_intersect_rays's result for it when that hit has t < tmax,
+ *     otherwise a miss (id -1, t -1, zeros).  A bound at or above FLT_MAX (+inf included) is no bound: NULL with tmax_all =
+ *     INFINITY is rtb_intersect_rays bit for bit.  A NaN bound, or one <= 0.0005 (the reference's least distance), is a miss.
+ *     The search starts at the bound, so the records' own strict `<` apply it: exact for PLANE, SPHERE, TRIANGLES and the
+ *     TUNNEL under every accelerator; a MESH record's hierarchy prunes against it, and its result is the masked unbounded one
+ *     except for rays whose winning pair lies in the grazing band (the mesh's contract, RTB_PRIM_MESH above).
+ *   RTB_QUERY_ANY: occluded[n] (required; the other outputs must be NULL) = 1 exactly when RTB_QUERY_CLOSEST with the same
+ *     bound would hit, else 0 (the grazing-band exception applies to meshes).  The walk stops at the first hit under the bound.
+ * Enqueued on `stream` (0 = the context's stream, not ordered with the legacy default stream: pass cudaStreamLegacy for that)
+ * behind the scene's upload and mesh updates; queries on different streams are ordered among themselves, and later mesh
+ * updates and rtb_scene_free wait for them.  Renders are not ordered against queries (both only read the scene).
+ * Checks come before anything is enqueued, and a refused call writes nothing: host memory, memory of another device, a
+ * misaligned buffer, n < 0, unknown flags or outputs that do not match them are RTB_ERR_INVALID.  n == 0 does nothing.   */
+enum { RTB_QUERY_CLOSEST = 0, RTB_QUERY_ANY = 1 };
+int rtb_query_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *rays, const float *tmax, float tmax_all,
+                   int32_t flags, int32_t *hit_id, float *hit_t, float *position, float *normal, uint8_t *occluded,
+                   void *stream);
+
 /* Replaces the ray loop of the reference's PerformanceTest console benchmark
  * (src/PerformanceTest/main.cpp:29-59 `trace`, 151-162): every ray of the batch [n][6] (HOST) is
  * mirror-reflected off whatever it hits until it reaches a PLANE geometry (the plane closing the tunnel

@@ -25,6 +25,7 @@ IPC_HANDLE_BYTES = 64
 PRIM_PLANE, PRIM_SPHERE, PRIM_TRIANGLES, PRIM_TUNNEL, PRIM_MESH = 0, 1, 2, 3, 4  # rtb_prim.type
 MESH_REBUILD, MESH_REFIT = 0, 1  # rtb_scene_mesh_update flags
 CUDA_STREAM_LEGACY = 1  # cudaStreamLegacy
+QUERY_CLOSEST, QUERY_ANY = 0, 1  # rtb_query_rays flags
 
 
 class RtbError(RuntimeError):
@@ -140,7 +141,7 @@ ABI_SYMBOLS = ["rtb_init", "rtb_shutdown", "rtb_last_error", "rtb_abi_version", 
                "rtb_device_alloc", "rtb_device_free", "rtb_device_download", "rtb_ipc_export", "rtb_ipc_open", "rtb_ipc_close", "rtb_scatter_shard_device",
                "rtb_multi_init", "rtb_multi_shutdown", "rtb_multi_count", "rtb_multi_ctx", "rtb_multi_last_error",
                "rtb_multi_scene_upload", "rtb_multi_scene_free", "rtb_multi_scene_upload_bytes", "rtb_multi_render",
-               "rtb_multi_scene_mesh_update"]
+               "rtb_multi_scene_mesh_update", "rtb_query_rays"]
 
 _cuda = None
 _host = None
@@ -185,6 +186,7 @@ def cuda_lib():
         lib.rtb_unshard_cols_device.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, vp]
         lib.rtb_trace_primary.argtypes = [vp, vp, C.POINTER(Camera), i32, i32, vp, vp, vp, vp, vp, i32]
         lib.rtb_intersect_rays.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp]
+        lib.rtb_query_rays.argtypes = [vp, vp, i64, vp, vp, C.c_float, i32, vp, vp, vp, vp, vp, vp]
         lib.rtb_forget_schedule.argtypes = [vp]
         lib.rtb_device_alloc.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
         lib.rtb_device_free.argtypes = [vp, vp]
@@ -785,6 +787,53 @@ class DeviceScene:
                                                          ht.ctypes.data, pos.ctypes.data, nrm.ctypes.data),
                         "rtb_intersect_rays")
         return hid, ht, pos, nrm
+
+    def query(self, rays, tmax=None, any_hit=False, stream=None, out=None):
+        """rtb_query_rays: closest hits under a strict per-ray distance bound, or occlusion (include/rtb.h), on the device and
+        ordered on `stream` with no host synchronisation.  `rays` is a contiguous CUDA float32 tensor [n][6] (origin, direction)
+        on the context's device; `tmax` None (no bound), a float, or a contiguous CUDA float32 tensor [n].  `stream` as in
+        mesh_update: torch's current stream by default.  The outputs are allocated on that stream, or taken from `out`:
+        closest: (hit_id int32 [n], hit_t float32 [n], position float32 [n][3], normal float32 [n][3]), any of them may be
+        None; any_hit: a torch.bool tensor [n] (True: something lies on the ray before tmax)."""
+        import torch
+        dev = torch.device("cuda", self.ctx.device)
+        if not (isinstance(rays, torch.Tensor) and rays.device == dev and rays.dtype == torch.float32 and rays.is_contiguous()
+                and rays.dim() == 2 and rays.shape[1] == 6):
+            raise RtbError(f"query: rays must be a contiguous float32 tensor [n][6] on {dev}")
+        n = rays.shape[0]
+        bound, tmax_all = None, float("inf")
+        if isinstance(tmax, torch.Tensor):
+            if tmax.device != dev or tmax.dtype != torch.float32 or not tmax.is_contiguous() or tuple(tmax.shape) != (n,):
+                raise RtbError(f"query: a tmax tensor must be a contiguous float32 tensor [n] on {dev}")
+            bound = tmax
+        elif tmax is not None:
+            tmax_all = float(tmax)
+        if stream is None:
+            stream = torch.cuda.current_stream(dev).cuda_stream or CUDA_STREAM_LEGACY  # see mesh_update
+        alloc_stream = torch.cuda.ExternalStream(stream, device=dev) if stream not in (0, CUDA_STREAM_LEGACY) else \
+            (torch.cuda.default_stream(dev) if stream == CUDA_STREAM_LEGACY else torch.cuda.current_stream(dev))
+        specs = [((n,), torch.bool)] if any_hit else [((n,), torch.int32), ((n,), torch.float32), ((n, 3), torch.float32),
+                                                     ((n, 3), torch.float32)]
+        if n == 0 and out is None:
+            return torch.zeros(0, dtype=torch.bool, device=dev) if any_hit else \
+                tuple(torch.zeros(shape, dtype=dt, device=dev) for shape, dt in specs)
+        if out is None:
+            with torch.cuda.stream(alloc_stream):
+                outs = [torch.empty(shape, dtype=dt, device=dev) for shape, dt in specs]
+        else:
+            outs = [out] if any_hit else list(out)
+            if len(outs) != len(specs) or (any_hit and outs[0] is None):
+                raise RtbError("query: out must be a bool tensor (any_hit) or a 4-tuple (hit_id, hit_t, position, normal)")
+            for o, (shape, dt) in zip(outs, specs):
+                if o is not None and (not isinstance(o, torch.Tensor) or o.device != dev or o.dtype != dt or
+                                      tuple(o.shape) != shape or not o.is_contiguous()):
+                    raise RtbError(f"query: an output must be a contiguous {dt} tensor {list(shape)} on {dev}")
+        p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        args = [None, None, None, None, p(outs[0])] if any_hit else [p(o) for o in outs] + [None]
+        self.ctx._check(self.ctx._lib.rtb_query_rays(self.ctx._h, self._h, n, p(rays), p(bound), tmax_all,
+                                                     QUERY_ANY if any_hit else QUERY_CLOSEST, *args, C.c_void_p(stream or 0)),
+                        "rtb_query_rays")
+        return outs[0] if any_hit else tuple(outs)
 
 
 # ---- synthetic models -------------------------------------------------------------------------

@@ -260,6 +260,12 @@ struct rtb_scene
     std::vector<int> mesh_prims; // prims indices of the MESH records (rtb_scene_mesh_download)
     cudaEvent_t last_use = nullptr; // recorded after every launch that reads the scene
     cudaEvent_t ready = nullptr;    // recorded on ctx->stream behind the upload copies
+    // rtb_query_rays on the caller's stream: queries are chained among themselves (a query on another stream than the last one
+    // waits for it), so `query_use`, recorded behind every query kernel, covers them all.  Not last_use: a query recording it
+    // would hide a render still running on another stream, and renders do not wait for queries.
+    mutable cudaEvent_t query_use = nullptr;
+    mutable cudaStream_t query_stream = nullptr;
+    mutable bool queried = false;
     bool direct_sources = false;    // some copies read the caller's page-locked arrays: rtb_scene_free waits for `ready`
     int64_t grid_cells_used = 0, grid_refs = 0, grid_words = 0;
     int64_t kd_nodes = 0, kd_refs = 0; // k-d tree resident on the device (uploaded or built there)
@@ -1279,7 +1285,8 @@ static int sceneUpload(rtb_ctx *ctx, const rtb_flat_scene *f, rtb_scene **out, b
     DScene &d = s->d;
     memset(&d, 0, sizeof(d));
     if (cudaEventCreateWithFlags(&s->last_use, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&s->ready, cudaEventDisableTiming) != cudaSuccess)
+        cudaEventCreateWithFlags(&s->ready, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&s->query_use, cudaEventDisableTiming) != cudaSuccess)
     {
         rtb_scene_free(ctx, s);
         return fail(ctx, RTB_ERR_CUDA, "rtb_scene_upload: cudaEventCreate failed");
@@ -1467,12 +1474,14 @@ extern "C" int rtb_scene_free(rtb_ctx *ctx, rtb_scene *s)
         // copies straight out of the caller's page-locked arrays: the caller may reuse them once the scene is freed
         if (s->direct_sources && s->ready && cudaEventQuery(s->ready) != cudaSuccess) { cudaGetLastError(); cudaEventSynchronize(s->ready); }
         if (s->last_use) cudaStreamWaitEvent(ctx->stream, s->last_use, 0);
+        if (s->query_use) cudaStreamWaitEvent(ctx->stream, s->query_use, 0);
         for (void *p : s->allocs) cudaFreeAsync(p, ctx->stream);
     }
     else
         for (void *p : s->allocs) cudaFree(p);
     if (s->last_use) cudaEventDestroy(s->last_use);
     if (s->ready) cudaEventDestroy(s->ready);
+    if (s->query_use) cudaEventDestroy(s->query_use);
     delete s;
     return RTB_OK;
 }
@@ -1637,6 +1646,7 @@ static int meshUpdateEnqueue(rtb_ctx *ctx, rtb_scene *s, const std::vector<int> 
     // renders on other streams record last_use behind their kernels, and frames of a context run one after the other
     // (waitLastFrame): the last one covers them all
     CUDA_TRY(ctx, cudaStreamWaitEvent(st, s->last_use, 0));
+    CUDA_TRY(ctx, cudaStreamWaitEvent(st, s->query_use, 0)); // queries on any stream (chained: the last one covers them all)
     // every allocation comes before the first write to the scene: a failed one leaves the scene as it was
     struct RawGuard { void *p = nullptr; cudaStream_t st; ~RawGuard() { if (p) cudaFreeAsync(p, st); } } raw{nullptr, st};
     MeshScratch t;
@@ -2592,6 +2602,60 @@ extern "C" int rtb_trace_primary(rtb_ctx *ctx, const rtb_scene *scene, const rtb
     return RTB_OK;
 }
 
+static void launchQuery(const rtb_scene *scene, const QueryParams &Q, bool any, cudaStream_t st)
+{
+    const unsigned int blocks = (unsigned int)((Q.n + RTB_CTA_THREADS - 1) / RTB_CTA_THREADS);
+    if (scene->has_mesh)
+    {
+        if (any) k_query_rays<true, true><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+        else k_query_rays<true, false><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+    }
+    else if (any) k_query_rays<false, true><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+    else k_query_rays<false, false><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+}
+
+// A caller's buffer for rtb_query_rays: memory of the context's device or managed memory, `align`-byte aligned
+static bool deviceBuffer(const rtb_ctx *ctx, const void *p, uintptr_t align)
+{
+    cudaPointerAttributes attr;
+    const bool known = cudaPointerGetAttributes(&attr, p) == cudaSuccess;
+    cudaGetLastError();
+    if (!known || ((uintptr_t)p & (align - 1))) return false;
+    return attr.type == cudaMemoryTypeManaged || (attr.type == cudaMemoryTypeDevice && attr.device == ctx->device);
+}
+
+extern "C" int rtb_query_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *rays, const float *tmax, float tmax_all,
+                              int32_t flags, int32_t *hit_id, float *hit_t, float *position, float *normal, uint8_t *occluded,
+                              void *stream)
+{
+    if (!ctx || !scene || n < 0) return fail(ctx, RTB_ERR_INVALID, "rtb_query_rays: bad argument");
+    if (flags != RTB_QUERY_CLOSEST && flags != RTB_QUERY_ANY) return fail(ctx, RTB_ERR_INVALID, "rtb_query_rays: unknown flags");
+    const bool any = flags == RTB_QUERY_ANY;
+    if (any ? (!occluded || hit_id || hit_t || position || normal) : occluded != nullptr)
+        return fail(ctx, RTB_ERR_INVALID, "rtb_query_rays: the outputs do not match the flags (ANY: occluded only; CLOSEST: no occluded)");
+    if (n == 0) return RTB_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    if (!rays || !deviceBuffer(ctx, rays, 8))
+        return fail(ctx, RTB_ERR_INVALID, "rtb_query_rays: rays must be 8-byte aligned memory of the context's device or managed memory");
+    const void *bufs[6] = {tmax, hit_id, hit_t, position, normal, occluded};
+    const uintptr_t align[6] = {4, 4, 4, 4, 4, 1};
+    for (int b = 0; b < 6; b++)
+        if (bufs[b] && !deviceBuffer(ctx, bufs[b], align[b]))
+            return fail(ctx, RTB_ERR_INVALID, "rtb_query_rays: tmax and the outputs must be aligned memory of the context's device or managed memory");
+    const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+    if (st != ctx->stream) CUDA_TRY(ctx, cudaStreamWaitEvent(st, scene->ready, 0)); // uploads and updates run on ctx->stream
+    if (scene->queried && st != scene->query_stream) CUDA_TRY(ctx, cudaStreamWaitEvent(st, scene->query_use, 0));
+    QueryParams Q = {};
+    Q.n = (long long)n; Q.rays = rays; Q.tmax = tmax; Q.tmax_all = tmax_all;
+    Q.hit_id = hit_id; Q.hit_t = hit_t; Q.position = position; Q.normal = normal; Q.occluded = occluded;
+    launchQuery(scene, Q, any, st);
+    CUDA_TRY(ctx, cudaGetLastError());
+    CUDA_TRY(ctx, cudaEventRecord(scene->query_use, st));
+    scene->query_stream = st;
+    scene->queried = true;
+    return RTB_OK;
+}
+
 extern "C" int rtb_intersect_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *rays, int32_t *hit_id,
                                   float *hit_t, float *position, float *normal)
 {
@@ -2606,9 +2670,10 @@ extern "C" int rtb_intersect_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t 
     if (hit_t) CUDA_TRY(ctx, d_t.alloc((size_t)n));
     if (position) CUDA_TRY(ctx, d_pos.alloc((size_t)n * 3));
     if (normal) CUDA_TRY(ctx, d_nrm.alloc((size_t)n * 3));
-    const unsigned int blocks = (unsigned int)((n + RTB_CTA_THREADS - 1) / RTB_CTA_THREADS);
-    if (scene->has_mesh) k_intersect_rays<true><<<blocks, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, (long long)n, d_rays.p, d_id.p, d_t.p, d_pos.p, d_nrm.p);
-    else k_intersect_rays<<<blocks, RTB_CTA_THREADS, 0, ctx->stream>>>(scene->d, (long long)n, d_rays.p, d_id.p, d_t.p, d_pos.p, d_nrm.p);
+    QueryParams Q = {};
+    Q.n = (long long)n; Q.rays = d_rays.p; Q.tmax_all = INFINITY;
+    Q.hit_id = d_id.p; Q.hit_t = d_t.p; Q.position = d_pos.p; Q.normal = d_nrm.p;
+    launchQuery(scene, Q, false, ctx->stream);
     CUDA_TRY(ctx, cudaGetLastError());
     if (hit_id) CUDA_TRY(ctx, cudaMemcpyAsync(hit_id, d_id.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     if (hit_t) CUDA_TRY(ctx, cudaMemcpyAsync(hit_t, d_t.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));

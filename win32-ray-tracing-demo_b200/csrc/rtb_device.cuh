@@ -669,8 +669,10 @@ __device__ bool convexIntersect(const DScene &S, const Ray &ray, RayCtx &ctx, in
 // Triangle mesh (RTB_PRIM_MESH): the hierarchy of rtb_build_bvh.cuh, nodes skipped by the test of rtb_bvh.h.  Nearest
 // accepted (t, k) in lexicographic order; `bestT` comes in as the nearest hit of the earlier records and `bestK` as -1, so
 // the mesh replaces it only with a strictly smaller t, as the run's `t < minDistance` does.  Visit order changes nothing.
+// ANY = true (occlusion queries): the walk ends at the first accepted triangle with t < bestT; bestT / bestK / nOut are then
+// that triangle's, not the nearest one's.
 // ---------------------------------------------------------------------------------------------
-template <class Probe>
+template <bool ANY = false, class Probe>
 __device__ bool meshIntersect(const DScene &S, unsigned int base, const Ray &ray, float &bestT, int &bestK, V3 &nOut, Probe &pr)
 {
     const rtb_bvh::Ray R = rtb_bvh::makeRay(ray.o.x, ray.o.y, ray.o.z, ray.d.x, ray.d.y, ray.d.z);
@@ -698,6 +700,7 @@ __device__ bool meshIntersect(const DScene &S, unsigned int base, const Ray &ray
         const bool h1 = c1 != c0 && rtb_bvh::nodeHit(R, lo1, hi1, bestT); // a one-triangle mesh links its leaf twice
         if (h0 && c0 < 0) leaf(~c0);
         if (h1 && c1 < 0) leaf(~c1);
+        if (ANY && found) break;
         const bool in0 = h0 && c0 >= 0, in1 = h1 && c1 >= 0;
         if (in0 && in1) { stack[sp++] = c1; node = c0; }
         else if (in0) node = c0;
@@ -717,14 +720,22 @@ struct Hit { int id; int mat; int prim_type; float t; V3 pos, n; };
 // earlier by the resumable traversal of rtb_chain_sm.cuh); everything else is evaluated here in
 // insertion order with the reference's strict `<`.
 // MESH = false: scenes without RTB_PRIM_MESH records (the kernels every other scene runs are compiled without the mesh walk)
-template <bool MESH = false, class Probe, class TunnelFn>
-__device__ __forceinline__ bool sceneIntersectWith(const DScene &S, const Ray &ray, Hit &best, Probe &pr, TunnelFn tunnel)
+// `start`: the search starts there instead of at FLT_MAX, so every record's strict `<` rejects hits at t >= start (the
+// bounded queries of rtb_query_rays; callers pass at most FLT_MAX).
+// ANY = true: occlusion -- true as soon as one record has a hit with t < start (the minimum over the records is below start
+// then, whatever the others hold); `best` is not filled.  The records are taken in order with the tunnel last, the TRIANGLES
+// runs and the mesh walk stop at their first accepted triangle, the tunnel runs its closest walk (DESIGN 3d).
+template <bool MESH = false, bool ANY = false, class Probe, class TunnelFn>
+__device__ __forceinline__ bool sceneIntersectWith(const DScene &S, const Ray &ray, Hit &best, Probe &pr, TunnelFn tunnel,
+                                                   float start = FLT_MAX)
 {
-    float minDistance = FLT_MAX;
+    float minDistance = start;
     best.id = -1;
+    bool tunnelLast = false;
     for (int i = 0; i < S.n_prims; i++)
     {
         const rtb_prim &P = S.prims[i];
+        if (ANY && best.id >= 0) return true;
         if (P.type == RTB_PRIM_PLANE)
         {
             const V3 normal = v3(P.v[0], P.v[1], P.v[2]);
@@ -772,6 +783,7 @@ __device__ __forceinline__ bool sceneIntersectWith(const DScene &S, const Ray &r
                 float t;
                 if (triIntersect(T, ray, t) && t < minDistance)
                 {
+                    if (ANY) return true;
                     minDistance = t;
                     best.id = P.base_id + k; best.mat = P.material; best.n = triNormal(T); best.prim_type = RTB_PRIM_TRIANGLES;
                 }
@@ -781,11 +793,12 @@ __device__ __forceinline__ bool sceneIntersectWith(const DScene &S, const Ray &r
         {
             int k = -1;
             V3 n;
-            if (meshIntersect(S, (unsigned int)S.mesh_base[i], ray, minDistance, k, n, pr))
+            if (meshIntersect<ANY>(S, (unsigned int)S.mesh_base[i], ray, minDistance, k, n, pr))
             {
                 best.id = P.base_id + k; best.mat = P.material; best.n = n; best.prim_type = RTB_PRIM_MESH;
             }
         }
+        else if (ANY) tunnelLast = true;
         else
         {
             int tri = -1;
@@ -799,29 +812,38 @@ __device__ __forceinline__ bool sceneIntersectWith(const DScene &S, const Ray &r
             }
         }
     }
+    if (ANY)
+    {
+        if (best.id >= 0) return true;
+        if (!tunnelLast) return false;
+        int tri = -1;
+        float t;
+        V3 n;
+        return tunnel(tri, t, n) && t < minDistance;
+    }
     if (best.id < 0) return false;
     best.t = minDistance;
     best.pos = at(ray, minDistance);
     return true;
 }
 
-template <bool MESH = false, class Probe>
-__device__ bool sceneIntersect(const DScene &S, const Ray &ray, Hit &best, Probe &pr, RayCtx &ctx)
+template <bool MESH = false, bool ANY = false, class Probe>
+__device__ bool sceneIntersect(const DScene &S, const Ray &ray, Hit &best, Probe &pr, RayCtx &ctx, float start = FLT_MAX)
 {
-    return sceneIntersectWith<MESH>(S, ray, best, pr, [&](int &tri, float &t, V3 &n) {
+    return sceneIntersectWith<MESH, ANY>(S, ray, best, pr, [&](int &tri, float &t, V3 &n) {
         if (S.accel == RTB_ACCEL_REGULAR_GRID || S.accel == RTB_ACCEL_FLAT_GRID) return gridIntersect<false>(S, ray, tri, t, n, pr);
         if (S.accel == RTB_ACCEL_KD_MEDIAN || S.accel == RTB_ACCEL_KD_SAH) return kdIntersect<false>(S, ray, tri, t, n, pr);
         if (S.accel == RTB_ACCEL_CONVEX || S.accel == RTB_ACCEL_CONVEX_SIMPLE) return convexIntersect(S, ray, ctx, tri, t, n, pr);
         return linearIntersect(S, ray, tri, t, n, pr);
-    });
+    }, start);
 }
 // a ray generated by the camera or by a caller carries a fresh context
-template <bool MESH = false, class Probe>
-__device__ bool sceneIntersect(const DScene &S, const Ray &ray, Hit &best, Probe &pr)
+template <bool MESH = false, bool ANY = false, class Probe>
+__device__ bool sceneIntersect(const DScene &S, const Ray &ray, Hit &best, Probe &pr, float start = FLT_MAX)
 {
     RayCtx ctx;
     ctx.inTunnel = 0; ctx.segment = -1;
-    return sceneIntersect<MESH>(S, ray, best, pr, ctx);
+    return sceneIntersect<MESH, ANY>(S, ray, best, pr, ctx, start);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -222,23 +222,44 @@ k_trace_primary(const __grid_constant__ DScene S, const __grid_constant__ FrameP
         for (int i = pr.len; i < seq_cap; i++) seq_buf[p * seq_cap + i] = -1;
 }
 
-template <bool MESH = false>
+// Ray queries (rtb_query_rays, rtb_intersect_rays): one lane per ray, the ray [6] floats read as three 64-bit loads.  The
+// search starts at the ray's bound (rtb.h: a strict bound; at or above FLT_MAX it starts at FLT_MAX, as the unbounded search
+// does -- +inf would accept hits at an infinite distance the unbounded search rejects; NaN or <= 0.0005 is a miss, every
+// accepted t being >= 0.0005).  ANY: occluded[i] = 1 exactly when the closest query with the same bound hits.
+struct QueryParams
+{
+    long long n;
+    const float *rays, *tmax; // tmax: [n] per-ray bounds, or null: tmax_all for every ray
+    float tmax_all;
+    int *hit_id;
+    float *hit_t, *position, *normal;
+    uint8_t *occluded;
+};
+
+template <bool MESH, bool ANY>
 __global__ void __launch_bounds__(RTB_CTA_THREADS)
-k_intersect_rays(const __grid_constant__ DScene S, long long n, const float *__restrict__ rays, int *__restrict__ hit_id,
-                 float *__restrict__ hit_t, float *__restrict__ position, float *__restrict__ normal)
+k_query_rays(const __grid_constant__ DScene S, const __grid_constant__ QueryParams Q)
 {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+    if (i >= Q.n) return;
+    const float2 *rp = reinterpret_cast<const float2 *>(Q.rays) + 3 * i;
+    const float2 a = __ldg(rp), b = __ldg(rp + 1), c = __ldg(rp + 2);
     Ray r;
-    r.o = v3(rays[6 * i], rays[6 * i + 1], rays[6 * i + 2]);
-    r.d = v3(rays[6 * i + 3], rays[6 * i + 4], rays[6 * i + 5]);
+    r.o = v3(a.x, a.y, b.x);
+    r.d = v3(b.y, c.x, c.y);
+    const float bound = Q.tmax ? __ldg(Q.tmax + i) : Q.tmax_all;
     NoProbe pr;
     Hit h;
-    const bool ok = sceneIntersect<MESH>(S, r, h, pr);
-    if (hit_id) hit_id[i] = ok ? h.id : -1;
-    if (hit_t) hit_t[i] = ok ? h.t : -1.0f;
-    if (position) { position[3 * i] = ok ? h.pos.x : 0; position[3 * i + 1] = ok ? h.pos.y : 0; position[3 * i + 2] = ok ? h.pos.z : 0; }
-    if (normal) { normal[3 * i] = ok ? h.n.x : 0; normal[3 * i + 1] = ok ? h.n.y : 0; normal[3 * i + 2] = ok ? h.n.z : 0; }
+    const bool ok = bound > 0.0005f && sceneIntersect<MESH, ANY>(S, r, h, pr, fminf(bound, FLT_MAX));
+    if (ANY)
+    {
+        Q.occluded[i] = ok ? 1 : 0;
+        return;
+    }
+    if (Q.hit_id) Q.hit_id[i] = ok ? h.id : -1;
+    if (Q.hit_t) Q.hit_t[i] = ok ? h.t : -1.0f;
+    if (Q.position) { Q.position[3 * i] = ok ? h.pos.x : 0; Q.position[3 * i + 1] = ok ? h.pos.y : 0; Q.position[3 * i + 2] = ok ? h.pos.z : 0; }
+    if (Q.normal) { Q.normal[3 * i] = ok ? h.n.x : 0; Q.normal[3 * i + 1] = ok ? h.n.y : 0; Q.normal[3 * i + 2] = ok ? h.n.z : 0; }
 }
 
 // ---------------------------------------------------------------------------------------------
