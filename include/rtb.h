@@ -372,6 +372,29 @@ int rtb_query_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float 
                    int32_t flags, int32_t *hit_id, float *hit_t, float *position, float *normal, uint8_t *occluded,
                    void *stream);
 
+/* Closest-point queries on DEVICE buffers, stream-ordered like rtb_query_rays (no host synchronisation, no allocation): the
+ * nearest point on the scene's triangles within a per-point radius, for contact generation, clearance checks or distance
+ * sampling in a physics or robotics step.  points = [n][3], rmax = [n] per-point radii or NULL: rmax_all for every point;
+ * every buffer is memory of the context's device or managed memory, 4-byte aligned (near: 1-byte).
+ * Records considered: TRIANGLES and MESH records only, in prims order (a MESH record is walked through its hierarchy and
+ * returns what the run of the same triangles returns, bit for bit, with no exception).  PLANE, SPHERE and TUNNEL records are
+ * ignored (upload the tunnel's triangles as a mesh to include them); a scene without triangle records returns misses.
+ * Distance: csrc/rtb_closest.h, one function compiled identically for host and device; d2 = the squared distance from the
+ * point to its closest point q on the triangle.  The winner is the smallest d2: ties within a record go to the lowest k, across
+ * records to the earlier record.  The bound is STRICT and squared: a pair counts when d2 < fl(r * r); r = +inf is no bound,
+ * r <= 0 or NaN is a miss, and so is a NaN point.
+ *   RTB_QUERY_CLOSEST: hit_id (base_id + k), distance = sqrtf(d2), position = q, normal = the stored, unflipped normal (any
+ *     may be NULL; near must be NULL).  A miss writes -1, -1, zeros, zeros.
+ *   RTB_QUERY_ANY: near[n] (required; the other outputs must be NULL) = 1 exactly when RTB_QUERY_CLOSEST with the same radius
+ *     hits, else 0.  The search stops at the first triangle within the radius.
+ * Ordering and refusals as rtb_query_rays: enqueued on `stream` (0 = the context's stream) behind the scene's upload and mesh
+ * updates, ordered with the other queries, awaited by later mesh updates and rtb_scene_free; host memory, memory of another
+ * device, a misaligned buffer, n < 0, unknown flags or outputs that do not match them are RTB_ERR_INVALID, and a refused call
+ * writes nothing.  n == 0 does nothing.                                                                                    */
+int rtb_query_points(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *points, const float *rmax, float rmax_all,
+                     int32_t flags, int32_t *hit_id, float *distance, float *position, float *normal, uint8_t *near,
+                     void *stream);
+
 /* Replaces the ray loop of the reference's PerformanceTest console benchmark
  * (src/PerformanceTest/main.cpp:29-59 `trace`, 151-162): every ray of the batch [n][6] (HOST) is
  * mirror-reflected off whatever it hits until it reaches a PLANE geometry (the plane closing the tunnel

@@ -25,7 +25,7 @@ IPC_HANDLE_BYTES = 64
 PRIM_PLANE, PRIM_SPHERE, PRIM_TRIANGLES, PRIM_TUNNEL, PRIM_MESH = 0, 1, 2, 3, 4  # rtb_prim.type
 MESH_REBUILD, MESH_REFIT = 0, 1  # rtb_scene_mesh_update flags
 CUDA_STREAM_LEGACY = 1  # cudaStreamLegacy
-QUERY_CLOSEST, QUERY_ANY = 0, 1  # rtb_query_rays flags
+QUERY_CLOSEST, QUERY_ANY = 0, 1  # rtb_query_rays / rtb_query_points flags
 
 
 class RtbError(RuntimeError):
@@ -141,7 +141,7 @@ ABI_SYMBOLS = ["rtb_init", "rtb_shutdown", "rtb_last_error", "rtb_abi_version", 
                "rtb_device_alloc", "rtb_device_free", "rtb_device_download", "rtb_ipc_export", "rtb_ipc_open", "rtb_ipc_close", "rtb_scatter_shard_device",
                "rtb_multi_init", "rtb_multi_shutdown", "rtb_multi_count", "rtb_multi_ctx", "rtb_multi_last_error",
                "rtb_multi_scene_upload", "rtb_multi_scene_free", "rtb_multi_scene_upload_bytes", "rtb_multi_render",
-               "rtb_multi_scene_mesh_update", "rtb_query_rays"]
+               "rtb_multi_scene_mesh_update", "rtb_query_rays", "rtb_query_points"]
 
 _cuda = None
 _host = None
@@ -187,6 +187,7 @@ def cuda_lib():
         lib.rtb_trace_primary.argtypes = [vp, vp, C.POINTER(Camera), i32, i32, vp, vp, vp, vp, vp, i32]
         lib.rtb_intersect_rays.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp]
         lib.rtb_query_rays.argtypes = [vp, vp, i64, vp, vp, C.c_float, i32, vp, vp, vp, vp, vp, vp]
+        lib.rtb_query_points.argtypes = [vp, vp, i64, vp, vp, C.c_float, i32, vp, vp, vp, vp, vp, vp]
         lib.rtb_forget_schedule.argtypes = [vp]
         lib.rtb_device_alloc.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
         lib.rtb_device_free.argtypes = [vp, vp]
@@ -795,19 +796,33 @@ class DeviceScene:
         mesh_update: torch's current stream by default.  The outputs are allocated on that stream, or taken from `out`:
         closest: (hit_id int32 [n], hit_t float32 [n], position float32 [n][3], normal float32 [n][3]), any of them may be
         None; any_hit: a torch.bool tensor [n] (True: something lies on the ray before tmax)."""
+        return self._device_query(self.ctx._lib.rtb_query_rays, "query", rays, 6, "rays", tmax, "tmax", any_hit, stream, out,
+                                  "hit_id, hit_t, position, normal")
+
+    def closest_points(self, points, max_dist=None, any_hit=False, stream=None, out=None):
+        """rtb_query_points: the nearest point on the scene's TRIANGLES and MESH records within a strict per-point radius, or
+        whether one lies within it (include/rtb.h), on the device and ordered on `stream` with no host synchronisation.
+        `points` is a contiguous CUDA float32 tensor [n][3] on the context's device; `max_dist` None (no bound), a float, or a
+        contiguous CUDA float32 tensor [n].  Streams and outputs as in query: closest: (hit_id int32 [n], distance float32 [n],
+        position float32 [n][3], normal float32 [n][3]); any_hit: a torch.bool tensor [n] (True: a triangle lies within
+        max_dist)."""
+        return self._device_query(self.ctx._lib.rtb_query_points, "closest_points", points, 3, "points", max_dist, "max_dist",
+                                  any_hit, stream, out, "hit_id, distance, position, normal")
+
+    def _device_query(self, fn, what, inp, width, inp_name, bound_arg, bound_name, any_hit, stream, out, out_names):
         import torch
         dev = torch.device("cuda", self.ctx.device)
-        if not (isinstance(rays, torch.Tensor) and rays.device == dev and rays.dtype == torch.float32 and rays.is_contiguous()
-                and rays.dim() == 2 and rays.shape[1] == 6):
-            raise RtbError(f"query: rays must be a contiguous float32 tensor [n][6] on {dev}")
-        n = rays.shape[0]
-        bound, tmax_all = None, float("inf")
-        if isinstance(tmax, torch.Tensor):
-            if tmax.device != dev or tmax.dtype != torch.float32 or not tmax.is_contiguous() or tuple(tmax.shape) != (n,):
-                raise RtbError(f"query: a tmax tensor must be a contiguous float32 tensor [n] on {dev}")
-            bound = tmax
-        elif tmax is not None:
-            tmax_all = float(tmax)
+        if not (isinstance(inp, torch.Tensor) and inp.device == dev and inp.dtype == torch.float32 and inp.is_contiguous()
+                and inp.dim() == 2 and inp.shape[1] == width):
+            raise RtbError(f"{what}: {inp_name} must be a contiguous float32 tensor [n][{width}] on {dev}")
+        n = inp.shape[0]
+        bound, bound_all = None, float("inf")
+        if isinstance(bound_arg, torch.Tensor):
+            if bound_arg.device != dev or bound_arg.dtype != torch.float32 or not bound_arg.is_contiguous() or tuple(bound_arg.shape) != (n,):
+                raise RtbError(f"{what}: a {bound_name} tensor must be a contiguous float32 tensor [n] on {dev}")
+            bound = bound_arg
+        elif bound_arg is not None:
+            bound_all = float(bound_arg)
         if stream is None:
             stream = torch.cuda.current_stream(dev).cuda_stream or CUDA_STREAM_LEGACY  # see mesh_update
         alloc_stream = torch.cuda.ExternalStream(stream, device=dev) if stream not in (0, CUDA_STREAM_LEGACY) else \
@@ -823,16 +838,15 @@ class DeviceScene:
         else:
             outs = [out] if any_hit else list(out)
             if len(outs) != len(specs) or (any_hit and outs[0] is None):
-                raise RtbError("query: out must be a bool tensor (any_hit) or a 4-tuple (hit_id, hit_t, position, normal)")
+                raise RtbError(f"{what}: out must be a bool tensor (any_hit) or a 4-tuple ({out_names})")
             for o, (shape, dt) in zip(outs, specs):
                 if o is not None and (not isinstance(o, torch.Tensor) or o.device != dev or o.dtype != dt or
                                       tuple(o.shape) != shape or not o.is_contiguous()):
-                    raise RtbError(f"query: an output must be a contiguous {dt} tensor {list(shape)} on {dev}")
+                    raise RtbError(f"{what}: an output must be a contiguous {dt} tensor {list(shape)} on {dev}")
         p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
         args = [None, None, None, None, p(outs[0])] if any_hit else [p(o) for o in outs] + [None]
-        self.ctx._check(self.ctx._lib.rtb_query_rays(self.ctx._h, self._h, n, p(rays), p(bound), tmax_all,
-                                                     QUERY_ANY if any_hit else QUERY_CLOSEST, *args, C.c_void_p(stream or 0)),
-                        "rtb_query_rays")
+        self.ctx._check(fn(self.ctx._h, self._h, n, p(inp), p(bound), bound_all, QUERY_ANY if any_hit else QUERY_CLOSEST, *args,
+                           C.c_void_p(stream or 0)), fn.__name__)
         return outs[0] if any_hit else tuple(outs)
 
 

@@ -2614,7 +2614,7 @@ static void launchQuery(const rtb_scene *scene, const QueryParams &Q, bool any, 
     else k_query_rays<false, false><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
 }
 
-// A caller's buffer for rtb_query_rays: memory of the context's device or managed memory, `align`-byte aligned
+// A caller's buffer for rtb_query_rays / rtb_query_points: memory of the context's device or managed memory, `align`-byte aligned
 static bool deviceBuffer(const rtb_ctx *ctx, const void *p, uintptr_t align)
 {
     cudaPointerAttributes attr;
@@ -2622,6 +2622,36 @@ static bool deviceBuffer(const rtb_ctx *ctx, const void *p, uintptr_t align)
     cudaGetLastError();
     if (!known || ((uintptr_t)p & (align - 1))) return false;
     return attr.type == cudaMemoryTypeManaged || (attr.type == cudaMemoryTypeDevice && attr.device == ctx->device);
+}
+
+// The part rtb_query_rays and rtb_query_points share.  Before the launch (queryBegin): the buffer checks -- the input array
+// `in` (required) and the optional bound and outputs `bufs` -- and the ordering of the caller's stream behind the scene's
+// upload / updates and behind the last query on another stream.  After it (queryEnd): query_use recorded on that stream.
+// Every check comes before anything is enqueued.
+static int queryBegin(rtb_ctx *ctx, const rtb_scene *scene, const char *fn, const char *in_name, const void *in, uintptr_t in_align,
+                      const void *const bufs[6], const uintptr_t align[6], const char *bufs_name, void *stream, cudaStream_t &st)
+{
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    if (!in || !deviceBuffer(ctx, in, in_align))
+        return fail(ctx, RTB_ERR_INVALID, std::string(fn) + ": " + in_name + " must be " + std::to_string(in_align) +
+                                              "-byte aligned memory of the context's device or managed memory");
+    for (int b = 0; b < 6; b++)
+        if (bufs[b] && !deviceBuffer(ctx, bufs[b], align[b]))
+            return fail(ctx, RTB_ERR_INVALID, std::string(fn) + ": " + bufs_name +
+                                                  " must be aligned memory of the context's device or managed memory");
+    st = stream ? (cudaStream_t)stream : ctx->stream;
+    if (st != ctx->stream) CUDA_TRY(ctx, cudaStreamWaitEvent(st, scene->ready, 0)); // uploads and updates run on ctx->stream
+    if (scene->queried && st != scene->query_stream) CUDA_TRY(ctx, cudaStreamWaitEvent(st, scene->query_use, 0));
+    return RTB_OK;
+}
+
+static int queryEnd(rtb_ctx *ctx, const rtb_scene *scene, cudaStream_t st)
+{
+    CUDA_TRY(ctx, cudaGetLastError());
+    CUDA_TRY(ctx, cudaEventRecord(scene->query_use, st));
+    scene->query_stream = st;
+    scene->queried = true;
+    return RTB_OK;
 }
 
 extern "C" int rtb_query_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *rays, const float *tmax, float tmax_all,
@@ -2634,26 +2664,40 @@ extern "C" int rtb_query_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, c
     if (any ? (!occluded || hit_id || hit_t || position || normal) : occluded != nullptr)
         return fail(ctx, RTB_ERR_INVALID, "rtb_query_rays: the outputs do not match the flags (ANY: occluded only; CLOSEST: no occluded)");
     if (n == 0) return RTB_OK;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    if (!rays || !deviceBuffer(ctx, rays, 8))
-        return fail(ctx, RTB_ERR_INVALID, "rtb_query_rays: rays must be 8-byte aligned memory of the context's device or managed memory");
     const void *bufs[6] = {tmax, hit_id, hit_t, position, normal, occluded};
     const uintptr_t align[6] = {4, 4, 4, 4, 4, 1};
-    for (int b = 0; b < 6; b++)
-        if (bufs[b] && !deviceBuffer(ctx, bufs[b], align[b]))
-            return fail(ctx, RTB_ERR_INVALID, "rtb_query_rays: tmax and the outputs must be aligned memory of the context's device or managed memory");
-    const cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-    if (st != ctx->stream) CUDA_TRY(ctx, cudaStreamWaitEvent(st, scene->ready, 0)); // uploads and updates run on ctx->stream
-    if (scene->queried && st != scene->query_stream) CUDA_TRY(ctx, cudaStreamWaitEvent(st, scene->query_use, 0));
+    cudaStream_t st;
+    const int rc = queryBegin(ctx, scene, "rtb_query_rays", "rays", rays, 8, bufs, align, "tmax and the outputs", stream, st);
+    if (rc != RTB_OK) return rc;
     QueryParams Q = {};
     Q.n = (long long)n; Q.rays = rays; Q.tmax = tmax; Q.tmax_all = tmax_all;
     Q.hit_id = hit_id; Q.hit_t = hit_t; Q.position = position; Q.normal = normal; Q.occluded = occluded;
     launchQuery(scene, Q, any, st);
-    CUDA_TRY(ctx, cudaGetLastError());
-    CUDA_TRY(ctx, cudaEventRecord(scene->query_use, st));
-    scene->query_stream = st;
-    scene->queried = true;
-    return RTB_OK;
+    return queryEnd(ctx, scene, st);
+}
+
+extern "C" int rtb_query_points(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *points, const float *rmax,
+                                float rmax_all, int32_t flags, int32_t *hit_id, float *distance, float *position, float *normal,
+                                uint8_t *near, void *stream)
+{
+    if (!ctx || !scene || n < 0) return fail(ctx, RTB_ERR_INVALID, "rtb_query_points: bad argument");
+    if (flags != RTB_QUERY_CLOSEST && flags != RTB_QUERY_ANY) return fail(ctx, RTB_ERR_INVALID, "rtb_query_points: unknown flags");
+    const bool any = flags == RTB_QUERY_ANY;
+    if (any ? (!near || hit_id || distance || position || normal) : near != nullptr)
+        return fail(ctx, RTB_ERR_INVALID, "rtb_query_points: the outputs do not match the flags (ANY: near only; CLOSEST: no near)");
+    if (n == 0) return RTB_OK;
+    const void *bufs[6] = {rmax, hit_id, distance, position, normal, near};
+    const uintptr_t align[6] = {4, 4, 4, 4, 4, 1};
+    cudaStream_t st;
+    const int rc = queryBegin(ctx, scene, "rtb_query_points", "points", points, 4, bufs, align, "rmax and the outputs", stream, st);
+    if (rc != RTB_OK) return rc;
+    PointParams Q = {};
+    Q.n = (long long)n; Q.points = points; Q.rmax = rmax; Q.rmax_all = rmax_all;
+    Q.hit_id = hit_id; Q.distance = distance; Q.position = position; Q.normal = normal; Q.near = near;
+    const unsigned int blocks = (unsigned int)((Q.n + RTB_CTA_THREADS - 1) / RTB_CTA_THREADS);
+    if (any) k_query_points<true><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+    else k_query_points<false><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+    return queryEnd(ctx, scene, st);
 }
 
 extern "C" int rtb_intersect_rays(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *rays, int32_t *hit_id,

@@ -1,8 +1,10 @@
 // rtb_misc.cuh -- the non-template kernels of the library (sm_100a): tile-order counting sort, parity hooks
-// (primary rays with traversal recording, ray batches), the PerformanceTest bounce loop, frame un-sharding.
+// (primary rays with traversal recording, ray batches), ray and closest-point queries, the PerformanceTest bounce loop,
+// frame un-sharding.
 // Included by exactly one translation unit (rtb_abi.cu).
 #pragma once
 #include "rtb_kernels.cuh"
+#include "rtb_closest.h"
 
 namespace rtb {
 
@@ -260,6 +262,132 @@ k_query_rays(const __grid_constant__ DScene S, const __grid_constant__ QueryPara
     if (Q.hit_t) Q.hit_t[i] = ok ? h.t : -1.0f;
     if (Q.position) { Q.position[3 * i] = ok ? h.pos.x : 0; Q.position[3 * i + 1] = ok ? h.pos.y : 0; Q.position[3 * i + 2] = ok ? h.pos.z : 0; }
     if (Q.normal) { Q.normal[3 * i] = ok ? h.n.x : 0; Q.normal[3 * i + 1] = ok ? h.n.y : 0; Q.normal[3 * i + 2] = ok ? h.n.z : 0; }
+}
+
+// Point queries (rtb_query_points): the nearest point on the TRIANGLES and MESH records within a strict per-point radius
+// (include/rtb.h, DESIGN 3e).  Distances are rtb_closest.h's squared distances d2; a pair is accepted when d2 < best, best
+// starting at fl(r * r).
+struct PointParams
+{
+    long long n;
+    const float *points, *rmax; // rmax: [n] per-point radii, or null: rmax_all for every point
+    float rmax_all;
+    int *hit_id;
+    float *distance, *position, *normal;
+    uint8_t *near;
+};
+
+__device__ __forceinline__ float closestOf(const float4 *tris, unsigned int idx, const float p[3])
+{
+    const TriData T = loadTri(tris, idx);
+    const float t[9] = {T.q0.x, T.q0.y, T.q0.z, T.q0.w, T.q1.x, T.q1.y, T.q1.z, T.q1.w, T.q2.x};
+    float q[3];
+    return rtb_closest::closestPoint(p, t, q);
+}
+
+// The hierarchy of a MESH record, walked from the root: both children's box distances per step, the nearer child first, the
+// other pushed with its distance and dropped when popped above the current best.  Nearest (d2, k) in lexicographic order;
+// `best` comes in as the earlier records' nearest d2 (or the bound) and bestK as -1, so the mesh replaces it only with a
+// strictly smaller d2, as the run's `d2 < best` does.  A node with boxDist2 > best holds no winner (rtb_closest.h), so the
+// result is the run's whatever the tree's shape.  ANY: ends at the first accepted triangle.  Returns the leaf position won.
+template <bool ANY>
+__device__ int meshClosest(const DScene &S, unsigned int base, const float p[3], float &best, int &bestK)
+{
+    const float4 *nodes = S.mesh_nodes + 4ull * base;
+    int stackNode[RTB_BVH_STACK];
+    float stackDist[RTB_BVH_STACK];
+    int sp = 0, node = 0, won = -1;
+    auto leaf = [&](int pos) {
+        const float d2 = closestOf(S.mesh_tris, base + (unsigned int)pos, p);
+        if (!(d2 <= best)) return;
+        const int k = (int)__ldg(S.mesh_order + base + pos);
+        if (d2 < best || k < bestK) { best = d2; bestK = k; won = pos; }
+    };
+    while (true)
+    {
+        const float4 *q = nodes + 4ull * (unsigned int)node;
+        const float4 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2), q3 = __ldg(q + 3);
+        const float lo0[3] = {q0.x, q0.y, q0.z}, lo1[3] = {q0.w, q1.x, q1.y};
+        const float hi0[3] = {q1.z, q1.w, q2.x}, hi1[3] = {q2.y, q2.z, q2.w};
+        const int c0 = __float_as_int(q3.x), c1 = __float_as_int(q3.y);
+        const float b0 = rtb_closest::boxDist2(p, lo0, hi0);
+        const bool two = c1 != c0; // a one-triangle mesh links its leaf twice
+        const float b1 = two ? rtb_closest::boxDist2(p, lo1, hi1) : INFINITY;
+        if (c0 < 0 && b0 <= best) leaf(~c0);
+        if (two && c1 < 0 && b1 <= best) leaf(~c1);
+        if (ANY && won >= 0) break;
+        const bool in0 = c0 >= 0 && b0 <= best, in1 = c1 >= 0 && b1 <= best;
+        if (in0 && in1)
+        {
+            const bool first1 = b1 < b0;
+            stackNode[sp] = first1 ? c0 : c1;
+            stackDist[sp++] = first1 ? b0 : b1;
+            node = first1 ? c1 : c0;
+        }
+        else if (in0) node = c0;
+        else if (in1) node = c1;
+        else
+        {
+            while (sp > 0 && stackDist[sp - 1] > best) sp--;
+            if (sp == 0) break;
+            node = stackNode[--sp];
+        }
+    }
+    return won;
+}
+
+template <bool ANY>
+__global__ void __launch_bounds__(RTB_CTA_THREADS)
+k_query_points(const __grid_constant__ DScene S, const __grid_constant__ PointParams Q)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= Q.n) return;
+    const float p[3] = {__ldg(Q.points + 3 * i), __ldg(Q.points + 3 * i + 1), __ldg(Q.points + 3 * i + 2)};
+    const float r = Q.rmax ? __ldg(Q.rmax + i) : Q.rmax_all;
+    float best = r * r;
+    int id = -1;
+    const float4 *winner = nullptr; // the winning triangle's record
+    if (r > 0.0f && p[0] == p[0] && p[1] == p[1] && p[2] == p[2]) // NaN or r <= 0: a miss without a walk
+        for (int j = 0; j < S.n_prims; j++)
+        {
+            const rtb_prim &P = S.prims[j];
+            if (ANY && id >= 0) break;
+            if (P.type == RTB_PRIM_TRIANGLES)
+            {
+                for (int k = 0; k < P.count; k++)
+                {
+                    const float d2 = closestOf(S.loose, (unsigned int)(P.first + k), p);
+                    if (d2 < best)
+                    {
+                        best = d2; id = P.base_id + k; winner = S.loose + 3ull * (unsigned int)(P.first + k);
+                        if (ANY) break;
+                    }
+                }
+            }
+            else if (P.type == RTB_PRIM_MESH)
+            {
+                int k = -1;
+                const int pos = meshClosest<ANY>(S, (unsigned int)S.mesh_base[j], p, best, k);
+                if (pos >= 0) { id = P.base_id + k; winner = S.mesh_tris + 3ull * ((unsigned int)S.mesh_base[j] + (unsigned int)pos); }
+            }
+        }
+    if (ANY)
+    {
+        Q.near[i] = id >= 0 ? 1 : 0;
+        return;
+    }
+    float q[3] = {0.0f, 0.0f, 0.0f}, nrm[3] = {0.0f, 0.0f, 0.0f};
+    if (id >= 0)
+    { // the winner's closest point again: the same function on the same record, so the same bits as in the search
+        const TriData T = loadTri(winner, 0);
+        const float t[9] = {T.q0.x, T.q0.y, T.q0.z, T.q0.w, T.q1.x, T.q1.y, T.q1.z, T.q1.w, T.q2.x};
+        rtb_closest::closestPoint(p, t, q);
+        nrm[0] = T.q2.y; nrm[1] = T.q2.z; nrm[2] = T.q2.w;
+    }
+    if (Q.hit_id) Q.hit_id[i] = id;
+    if (Q.distance) Q.distance[i] = id >= 0 ? sqrtf(best) : -1.0f;
+    if (Q.position) { Q.position[3 * i] = q[0]; Q.position[3 * i + 1] = q[1]; Q.position[3 * i + 2] = q[2]; }
+    if (Q.normal) { Q.normal[3 * i] = nrm[0]; Q.normal[3 * i + 1] = nrm[1]; Q.normal[3 * i + 2] = nrm[2]; }
 }
 
 // ---------------------------------------------------------------------------------------------
