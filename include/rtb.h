@@ -395,6 +395,30 @@ int rtb_query_points(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const floa
                      int32_t flags, int32_t *hit_id, float *distance, float *position, float *normal, uint8_t *near,
                      void *stream);
 
+/* First-order moments of every MESH record's hierarchy, for rtb_query_winding: per node and child the area vector, the
+ * area-weighted centre and a radius about it (64 bytes per node slot; rtb_scene_device_bytes grows by 64 x the scene's mesh
+ * triangles).  Opt-in: rtb_scene_upload does not build them.  Once built, rtb_scene_mesh_update (rebuild and refit) keeps
+ * them current with no new allocation.  Ordered like rtb_scene_mesh_update: enqueued on the context's stream behind `stream`
+ * (0 = the context's stream) and every launch that has read the scene, and `stream` waits for it.  A second call, and a call
+ * on a scene without MESH records, does nothing.                                                                          */
+int rtb_scene_mesh_moments(rtb_ctx *ctx, rtb_scene *scene, void *stream);
+
+/* Winding-number queries on DEVICE buffers, stream-ordered like rtb_query_points: inside / outside tests for occupancy,
+ * penetration depth or SDF sampling.  points = [n][3]; winding = [n] float, inside = [n] uint8, either may be NULL but not
+ * both; every buffer is memory of the context's device or managed memory, 4-byte aligned (inside: 1-byte).
+ * winding[i] = the generalised winding number sum_t Omega_t(p) / 4 pi over the TRIANGLES and MESH records, in prims order
+ * (overlapping records count once each; PLANE, SPHERE and TUNNEL records are ignored): 1 inside and 0 outside a closed
+ * surface whose facets follow the right-hand rule outwards (the vertex order decides, never the stored normal), fractional
+ * for open soups.  inside[i] = winding[i] > 0.5.  Solid angles: csrc/rtb_winding.h, one function compiled identically for
+ * host and device.  A TRIANGLES run sums every triangle exactly, in k order.  A MESH record walks its hierarchy: a leaf adds
+ * its exact solid angle, an inner child whose centre lies farther than beta x its radius adds its dipole (Barill et al.
+ * 2018), any other child is descended into.  beta = +inf sums every triangle exactly; beta must be >= 1 (2 is the usual
+ * choice).  A NaN point gives NaN / 0.
+ * Refused with RTB_ERR_INVALID, writing nothing: n < 0, beta NaN or below 1, no output, a scene with MESH records but no
+ * moments (rtb_scene_mesh_moments), and the buffer refusals of rtb_query_points.  n == 0 does nothing.                     */
+int rtb_query_winding(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *points, float beta, float *winding,
+                      uint8_t *inside, void *stream);
+
 /* Replaces the ray loop of the reference's PerformanceTest console benchmark
  * (src/PerformanceTest/main.cpp:29-59 `trace`, 151-162): every ray of the batch [n][6] (HOST) is
  * mirror-reflected off whatever it hits until it reaches a PLANE geometry (the plane closing the tunnel

@@ -141,7 +141,8 @@ ABI_SYMBOLS = ["rtb_init", "rtb_shutdown", "rtb_last_error", "rtb_abi_version", 
                "rtb_device_alloc", "rtb_device_free", "rtb_device_download", "rtb_ipc_export", "rtb_ipc_open", "rtb_ipc_close", "rtb_scatter_shard_device",
                "rtb_multi_init", "rtb_multi_shutdown", "rtb_multi_count", "rtb_multi_ctx", "rtb_multi_last_error",
                "rtb_multi_scene_upload", "rtb_multi_scene_free", "rtb_multi_scene_upload_bytes", "rtb_multi_render",
-               "rtb_multi_scene_mesh_update", "rtb_query_rays", "rtb_query_points"]
+               "rtb_multi_scene_mesh_update", "rtb_query_rays", "rtb_query_points",
+               "rtb_scene_mesh_moments", "rtb_query_winding"]
 
 _cuda = None
 _host = None
@@ -188,6 +189,8 @@ def cuda_lib():
         lib.rtb_intersect_rays.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp]
         lib.rtb_query_rays.argtypes = [vp, vp, i64, vp, vp, C.c_float, i32, vp, vp, vp, vp, vp, vp]
         lib.rtb_query_points.argtypes = [vp, vp, i64, vp, vp, C.c_float, i32, vp, vp, vp, vp, vp, vp]
+        lib.rtb_scene_mesh_moments.argtypes = [vp, vp, vp]
+        lib.rtb_query_winding.argtypes = [vp, vp, i64, vp, C.c_float, vp, vp, vp]
         lib.rtb_forget_schedule.argtypes = [vp]
         lib.rtb_device_alloc.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
         lib.rtb_device_free.argtypes = [vp, vp]
@@ -676,6 +679,7 @@ class DeviceScene:
     def __init__(self, ctx, flat):
         self.ctx = ctx
         self._h = C.c_void_p()
+        self._moments = False  # rtb_scene_mesh_moments has run (winding_numbers builds them on first use)
         ctx._check(ctx._lib.rtb_scene_upload(ctx._h, flat, C.byref(self._h)), "rtb_scene_upload")
 
     def close(self):
@@ -823,10 +827,7 @@ class DeviceScene:
             bound = bound_arg
         elif bound_arg is not None:
             bound_all = float(bound_arg)
-        if stream is None:
-            stream = torch.cuda.current_stream(dev).cuda_stream or CUDA_STREAM_LEGACY  # see mesh_update
-        alloc_stream = torch.cuda.ExternalStream(stream, device=dev) if stream not in (0, CUDA_STREAM_LEGACY) else \
-            (torch.cuda.default_stream(dev) if stream == CUDA_STREAM_LEGACY else torch.cuda.current_stream(dev))
+        stream, alloc_stream = _query_stream(dev, stream)
         specs = [((n,), torch.bool)] if any_hit else [((n,), torch.int32), ((n,), torch.float32), ((n, 3), torch.float32),
                                                      ((n, 3), torch.float32)]
         if n == 0 and out is None:
@@ -848,6 +849,79 @@ class DeviceScene:
         self.ctx._check(fn(self.ctx._h, self._h, n, p(inp), p(bound), bound_all, QUERY_ANY if any_hit else QUERY_CLOSEST, *args,
                            C.c_void_p(stream or 0)), fn.__name__)
         return outs[0] if any_hit else tuple(outs)
+
+    def mesh_moments(self, stream=None):
+        """rtb_scene_mesh_moments: build the first-order moments of every mesh hierarchy (include/rtb.h), which winding
+        queries on a scene with MESH records need; winding_numbers, contains and signed_distance call it on first use.
+        `stream` as in mesh_update (torch's current stream by default).  A second call does nothing."""
+        if self._moments:
+            return
+        if stream is None:
+            import torch
+            stream = torch.cuda.current_stream(torch.device("cuda", self.ctx.device)).cuda_stream or CUDA_STREAM_LEGACY
+        self.ctx._check(self.ctx._lib.rtb_scene_mesh_moments(self.ctx._h, self._h, C.c_void_p(stream or 0)), "rtb_scene_mesh_moments")
+        self._moments = True
+
+    def winding_numbers(self, points, beta=2.0, stream=None, out=None):
+        """rtb_query_winding: the generalised winding number of every point with respect to the scene's TRIANGLES and MESH
+        records (include/rtb.h), on the device and ordered on `stream` with no host synchronisation: about 1 inside and 0
+        outside a closed, outward-oriented surface.  `points` is a contiguous CUDA float32 tensor [n][3] on the context's
+        device; beta >= 1 trades accuracy for speed on meshes (+inf: exact).  Streams and `out` (a float32 tensor [n]) as in
+        query.  The first call builds the mesh moments (mesh_moments) on the same stream."""
+        return self._winding(points, beta, stream, out, False)
+
+    def contains(self, points, beta=2.0, stream=None, out=None):
+        """rtb_query_winding's inside test: a torch.bool tensor [n], True where winding_numbers(points, beta) > 0.5."""
+        return self._winding(points, beta, stream, out, True)
+
+    def signed_distance(self, points, max_dist=None, beta=2.0, stream=None):
+        """closest_points with the sign of contains: (signed distance float32 [n], hit_id, position, normal).  The distance is
+        closest_points' distance, negated where contains(points, beta) is True; a point with no triangle within max_dist gets
+        -inf inside and +inf outside.  Two launches on one stream, combined by torch elementwise ops on that stream."""
+        import torch
+        dev = torch.device("cuda", self.ctx.device)
+        stream, alloc_stream = _query_stream(dev, stream)
+        hit_id, dist, pos, nrm = self.closest_points(points, max_dist, stream=stream)
+        ins = self.contains(points, beta, stream=stream)
+        with torch.cuda.stream(alloc_stream):
+            sd = torch.where(hit_id >= 0, dist, float("inf"))
+            sd = torch.where(ins, -sd, sd)
+        return sd, hit_id, pos, nrm
+
+    def _winding(self, points, beta, stream, out, inside):
+        import torch
+        dev = torch.device("cuda", self.ctx.device)
+        what = "contains" if inside else "winding_numbers"
+        if not (isinstance(points, torch.Tensor) and points.device == dev and points.dtype == torch.float32 and points.is_contiguous()
+                and points.dim() == 2 and points.shape[1] == 3):
+            raise RtbError(f"{what}: points must be a contiguous float32 tensor [n][3] on {dev}")
+        n = points.shape[0]
+        stream, alloc_stream = _query_stream(dev, stream)
+        dt = torch.bool if inside else torch.float32
+        if out is None:
+            with torch.cuda.stream(alloc_stream):
+                out = torch.empty(n, dtype=dt, device=dev)
+        elif not (isinstance(out, torch.Tensor) and out.device == dev and out.dtype == dt and tuple(out.shape) == (n,) and out.is_contiguous()):
+            raise RtbError(f"{what}: out must be a contiguous {dt} tensor [{n}] on {dev}")
+        if n == 0:
+            return out
+        self.mesh_moments(stream)
+        p = C.c_void_p(out.data_ptr())
+        self.ctx._check(self.ctx._lib.rtb_query_winding(self.ctx._h, self._h, n, C.c_void_p(points.data_ptr()), float(beta),
+                                                        None if inside else p, p if inside else None, C.c_void_p(stream or 0)),
+                        "rtb_query_winding")
+        return out
+
+
+def _query_stream(dev, stream):
+    """(handle, torch stream) of a query: torch's current stream by default (cudaStreamLegacy for its default stream: see
+    DeviceScene.mesh_update); the torch stream is the one outputs are allocated on."""
+    import torch
+    if stream is None:
+        stream = torch.cuda.current_stream(dev).cuda_stream or CUDA_STREAM_LEGACY
+    alloc_stream = torch.cuda.ExternalStream(stream, device=dev) if stream not in (0, CUDA_STREAM_LEGACY) else \
+        (torch.cuda.default_stream(dev) if stream == CUDA_STREAM_LEGACY else torch.cuda.current_stream(dev))
+    return stream, alloc_stream
 
 
 # ---- synthetic models -------------------------------------------------------------------------

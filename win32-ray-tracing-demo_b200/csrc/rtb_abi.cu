@@ -258,6 +258,9 @@ struct rtb_scene
     bool has_tunnel = false;
     bool has_mesh = false;   // RTB_PRIM_MESH records: the MESH kernel instantiations, no tunnel tiers
     std::vector<int> mesh_prims; // prims indices of the MESH records (rtb_scene_mesh_download)
+    // first-order moments of every mesh node slot (rtb_scene_mesh_moments, 4 float4 per slot, parallel to DScene::mesh_nodes):
+    // null until that call; kept out of DScene so that no other kernel's parameters change
+    const float4 *mesh_moments = nullptr;
     cudaEvent_t last_use = nullptr; // recorded after every launch that reads the scene
     cudaEvent_t ready = nullptr;    // recorded on ctx->stream behind the upload copies
     // rtb_query_rays on the caller's stream: queries are chained among themselves (a query on another stream than the last one
@@ -1179,7 +1182,7 @@ struct MeshScratch
     int *parent = nullptr; // inner nodes' links at [0, maxN), leaves' at [maxN, 2 maxN)
     void *tmp = nullptr;
     std::vector<void *> temps;
-    // rebuild = false: only what a refit uses (arrivals and parent links)
+    // rebuild = false: only what a refit or the moments use (arrivals and parent links)
     cudaError_t alloc(cudaStream_t stream, size_t n, bool rebuild)
     {
         st = stream;
@@ -1198,9 +1201,25 @@ struct MeshScratch
     ~MeshScratch() { for (void *p : temps) cudaFreeAsync(p, st); }
 };
 
+// The moments of MESH record i (k_bvh_moments) into `moments` (the scene's array, 4 float4 per node slot) from its leaf-order
+// records and its tree; the parent links in `t` must be the tree's (k_bvh_hierarchy or k_bvh_parents wrote them).  Uses the
+// arrival counters of `t` and allocates nothing.
+static int meshMoments(rtb_ctx *ctx, const rtb_scene *s, int i, MeshScratch &t, float4 *moments)
+{
+    const DScene &d = s->d;
+    const int n = d.prims[i].count;
+    const unsigned int tb = 256, nb = (unsigned int)((n + tb - 1) / tb);
+    const size_t base = (size_t)d.mesh_base[i];
+    CUDA_TRY(ctx, cudaMemsetAsync(t.arrivals, 0, (size_t)n * sizeof(unsigned int), t.st));
+    k_bvh_moments<<<nb, tb, 0, t.st>>>(d.mesh_tris + 3 * base, n, reinterpret_cast<const rtb_bvhnode *>(d.mesh_nodes) + base, t.parent,
+                                       t.parent + t.maxN, t.arrivals, reinterpret_cast<float *>(moments + 4 * base));
+    CUDA_TRY(ctx, cudaGetLastError());
+    return RTB_OK;
+}
+
 // The hierarchy of MESH record i from its raw records `raw` ([count][12] on the device) and its packed records, already in
 // DScene::loose.  rebuild: the whole LBVH pipeline (what rtb_scene_upload runs); otherwise a refit: child links and leaf
-// order are kept, every box is computed again from the new records.
+// order are kept, every box is computed again from the new records.  Moments, once the scene has them, follow either way.
 static int meshRecord(rtb_ctx *ctx, rtb_scene *s, int i, const float *raw, MeshScratch &t, bool rebuild)
 {
     DScene &d = s->d;
@@ -1227,7 +1246,7 @@ static int meshRecord(rtb_ctx *ctx, rtb_scene *s, int i, const float *raw, MeshS
     k_bvh_boxes<<<nb, tb, 0, st>>>(raw, order, n, nodes, t.parent, t.parent + t.maxN, t.arrivals);
     k_bvh_leaves<<<nb, tb, 0, st>>>(d.loose + 3ull * (unsigned int)P.first, order, n, const_cast<float4 *>(d.mesh_tris) + 3 * base);
     CUDA_TRY(ctx, cudaGetLastError());
-    return RTB_OK;
+    return s->mesh_moments ? meshMoments(ctx, s, i, t, const_cast<float4 *>(s->mesh_moments)) : RTB_OK;
 }
 
 // Hierarchies of the MESH records (rtb_build_bvh.cuh) from the raw loose records on the device.  Every record gets its own
@@ -1698,6 +1717,58 @@ extern "C" int rtb_scene_mesh_update(rtb_ctx *ctx, rtb_scene *s, int32_t mesh_in
         src = (const float *)staged;
     }
     return meshUpdateEnqueue(ctx, s, recs, src, !onDevice, flags, stream ? (cudaStream_t)stream : ctx->stream);
+}
+
+extern "C" int rtb_scene_mesh_moments(rtb_ctx *ctx, rtb_scene *s, void *stream)
+{
+    if (!ctx || !s) return fail(ctx, RTB_ERR_INVALID, "rtb_scene_mesh_moments: null argument");
+    if (s->mesh_moments || s->mesh_prims.empty()) return RTB_OK; // built already, or nothing to build
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const DScene &d = s->d;
+    const cudaStream_t st = ctx->stream, caller = stream ? (cudaStream_t)stream : st;
+    size_t slots = 0, maxN = 0;
+    for (int i : s->mesh_prims)
+    {
+        slots += (size_t)d.prims[i].count;
+        maxN = std::max(maxN, (size_t)d.prims[i].count);
+    }
+    // ordered as a mesh update: behind the caller's stream and every launch that has read the scene
+    if (caller != st)
+    {
+        if (!ctx->caller_ready) CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->caller_ready, cudaEventDisableTiming));
+        CUDA_TRY(ctx, cudaEventRecord(ctx->caller_ready, caller));
+        CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->caller_ready, 0));
+    }
+    CUDA_TRY(ctx, cudaStreamWaitEvent(st, s->last_use, 0));
+    CUDA_TRY(ctx, cudaStreamWaitEvent(st, s->query_use, 0));
+    MeshScratch t;
+    CUDA_TRY(ctx, t.alloc(st, maxN, false));
+    float4 *moments = nullptr;
+    int rc = deviceArray(ctx, s, 4 * slots, &moments, true);
+    if (rc != RTB_OK) return rc;
+    // the scene has moments only once every launch is enqueued: a failed call releases the array and leaves the scene without
+    // them, so a query stays refused and a later call builds them again
+    auto failed = [&](int code) {
+        s->allocs.pop_back();
+        s->bytes -= (int64_t)(4 * slots * sizeof(float4));
+        cudaFreeAsync(moments, st);
+        return code;
+    };
+    cudaError_t e = cudaMemsetAsync(moments, 0, 4 * slots * sizeof(float4), st);
+    if (e != cudaSuccess) return failed(fail(ctx, RTB_ERR_CUDA, std::string("rtb_scene_mesh_moments: ") + cudaGetErrorString(e)));
+    for (int i : s->mesh_prims)
+    {
+        const int n = d.prims[i].count;
+        if (n > 1)
+            k_bvh_parents<<<(unsigned int)((n - 1 + 255) / 256), 256, 0, st>>>(reinterpret_cast<const rtb_bvhnode *>(d.mesh_nodes) + d.mesh_base[i],
+                                                                              n, t.parent, t.parent + t.maxN);
+        if ((rc = meshMoments(ctx, s, i, t, moments)) != RTB_OK) return failed(rc);
+    }
+    if ((e = cudaEventRecord(s->ready, st)) != cudaSuccess ||
+        (caller != st && (e = cudaStreamWaitEvent(caller, s->ready, 0)) != cudaSuccess))
+        return failed(fail(ctx, RTB_ERR_CUDA, std::string("rtb_scene_mesh_moments: ") + cudaGetErrorString(e)));
+    s->mesh_moments = moments;
+    return RTB_OK;
 }
 
 // ---- render -----------------------------------------------------------------------------------
@@ -2614,7 +2685,7 @@ static void launchQuery(const rtb_scene *scene, const QueryParams &Q, bool any, 
     else k_query_rays<false, false><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
 }
 
-// A caller's buffer for rtb_query_rays / rtb_query_points: memory of the context's device or managed memory, `align`-byte aligned
+// A caller's buffer for rtb_query_rays / rtb_query_points / rtb_query_winding: memory of the context's device or managed memory, `align`-byte aligned
 static bool deviceBuffer(const rtb_ctx *ctx, const void *p, uintptr_t align)
 {
     cudaPointerAttributes attr;
@@ -2624,7 +2695,7 @@ static bool deviceBuffer(const rtb_ctx *ctx, const void *p, uintptr_t align)
     return attr.type == cudaMemoryTypeManaged || (attr.type == cudaMemoryTypeDevice && attr.device == ctx->device);
 }
 
-// The part rtb_query_rays and rtb_query_points share.  Before the launch (queryBegin): the buffer checks -- the input array
+// The part rtb_query_rays, rtb_query_points and rtb_query_winding share.  Before the launch (queryBegin): the buffer checks -- the input array
 // `in` (required) and the optional bound and outputs `bufs` -- and the ordering of the caller's stream behind the scene's
 // upload / updates and behind the last query on another stream.  After it (queryEnd): query_use recorded on that stream.
 // Every check comes before anything is enqueued.
@@ -2697,6 +2768,27 @@ extern "C" int rtb_query_points(rtb_ctx *ctx, const rtb_scene *scene, int64_t n,
     const unsigned int blocks = (unsigned int)((Q.n + RTB_CTA_THREADS - 1) / RTB_CTA_THREADS);
     if (any) k_query_points<true><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
     else k_query_points<false><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+    return queryEnd(ctx, scene, st);
+}
+
+extern "C" int rtb_query_winding(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *points, float beta, float *winding,
+                                 uint8_t *inside, void *stream)
+{
+    if (!ctx || !scene || n < 0) return fail(ctx, RTB_ERR_INVALID, "rtb_query_winding: bad argument");
+    if (!(beta >= 1.0f)) return fail(ctx, RTB_ERR_INVALID, "rtb_query_winding: beta must be >= 1 (+inf: exact)");
+    if (!winding && !inside) return fail(ctx, RTB_ERR_INVALID, "rtb_query_winding: no output (winding and inside are both null)");
+    if (!scene->mesh_prims.empty() && !scene->mesh_moments)
+        return fail(ctx, RTB_ERR_INVALID, "rtb_query_winding: the scene has MESH records but no moments: call rtb_scene_mesh_moments first");
+    if (n == 0) return RTB_OK;
+    const void *bufs[6] = {winding, inside, nullptr, nullptr, nullptr, nullptr};
+    const uintptr_t align[6] = {4, 1, 1, 1, 1, 1};
+    cudaStream_t st;
+    const int rc = queryBegin(ctx, scene, "rtb_query_winding", "points", points, 4, bufs, align, "the outputs", stream, st);
+    if (rc != RTB_OK) return rc;
+    WindingParams Q = {};
+    Q.n = (long long)n; Q.points = points; Q.moments = scene->mesh_moments; Q.beta = beta;
+    Q.winding = winding; Q.inside = inside;
+    k_query_winding<<<(unsigned int)((Q.n + RTB_CTA_THREADS - 1) / RTB_CTA_THREADS), RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
     return queryEnd(ctx, scene, st);
 }
 

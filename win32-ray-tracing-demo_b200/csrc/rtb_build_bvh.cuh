@@ -12,9 +12,11 @@
 // Every step is a deterministic function of the input: two builds of the same mesh are byte-identical.
 // A refit (rtb_scene_mesh_update) keeps the child links and the leaf order: it derives the parent links from the child links
 // (k_bvh_parents) and runs steps 6 and 7 again on the new records.
+// Moments (k_bvh_moments, opt-in through rtb_scene_mesh_moments) follow step 7, after a build, a refit or a rebuild alike.
 #pragma once
 #include <cub/cub.cuh>
 #include "rtb_bvh.h"
+#include "rtb_winding.h"
 
 namespace rtb {
 
@@ -176,6 +178,64 @@ __global__ void k_bvh_leaves(const float4 *__restrict__ exact, const uint32_t *_
     if (p >= n) return;
     const unsigned int k = leaf_order[p];
     for (int j = 0; j < 3; j++) leaf_tris[3ull * p + j] = exact[3ull * k + j];
+}
+
+// First-order moments of the winding queries (rtb_scene_mesh_moments), 16 floats per node slot, parallel to the nodes:
+// {N0, c0, r0, N1, c1, r1, 0, 0} -- per child the area vector, the area-weighted centre and a radius about it that holds
+// every vertex below.  Bottom-up with the arrival scheme of k_bvh_boxes, from the leaf-order records of k_bvh_leaves; the
+// second thread to reach a node combines its two slots in child order, so the result does not depend on the arrival order.
+__global__ void k_bvh_moments(const float4 *__restrict__ leaf_tris, int n, const rtb_bvhnode *__restrict__ nodes,
+                              const int *__restrict__ parent_inner, const int *__restrict__ parent_leaf,
+                              unsigned int *__restrict__ arrivals, float *__restrict__ moments)
+{
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n) return;
+    float t[12], N[3], c[3], r;
+    for (int j = 0; j < 3; j++)
+    {
+        const float4 q = leaf_tris[3ull * p + j];
+        t[4 * j] = q.x; t[4 * j + 1] = q.y; t[4 * j + 2] = q.z; t[4 * j + 3] = q.w;
+    }
+    rtb_winding::triMoment(t, N, c, r);
+    auto store = [&](float *m) { m[0] = N[0]; m[1] = N[1]; m[2] = N[2]; m[3] = c[0]; m[4] = c[1]; m[5] = c[2]; m[6] = r; };
+    if (n == 1)
+    { // a single leaf: both slots of the root hold it
+        store(moments);
+        store(moments + 7);
+        return;
+    }
+    int slot = parent_leaf[p];
+    while (true)
+    {
+        const int node = slot >> 1, side = slot & 1;
+        float *m = moments + 16ull * node;
+        store(m + 7 * side);
+        __threadfence();
+        if (atomicAdd(arrivals + node, 1u) == 0u) return; // the sibling is still on its way: it continues
+        __threadfence();
+        float s[14];
+        for (int j = 0; j < 14; j++) s[j] = __ldcg(m + j);
+        const float *N0 = s, *c0 = s + 3, *N1 = s + 7, *c1 = s + 10;
+        const float a0 = rtb_winding::norm3(N0), a1 = rtb_winding::norm3(N1), a = a0 + a1;
+        for (int i = 0; i < 3; i++) N[i] = N0[i] + N1[i];
+        if (a > 0.0f)
+            for (int i = 0; i < 3; i++) c[i] = (c0[i] * a0 + c1[i] * a1) / a;
+        else
+        { // no area below: the centre of the node's box
+            const rtb_bvhnode &b = nodes[node];
+            for (int i = 0; i < 3; i++)
+            {
+                const float lo = b.lo[0][i] < b.lo[1][i] ? b.lo[0][i] : b.lo[1][i];
+                const float hi = b.hi[0][i] > b.hi[1][i] ? b.hi[0][i] : b.hi[1][i];
+                c[i] = (lo + hi) * 0.5f;
+            }
+        }
+        const float d0[3] = {c[0] - c0[0], c[1] - c0[1], c[2] - c0[2]}, d1[3] = {c[0] - c1[0], c[1] - c1[1], c[2] - c1[2]};
+        const float r0 = rtb_winding::norm3(d0) + s[6], r1 = rtb_winding::norm3(d1) + s[13];
+        r = (r0 > r1 ? r0 : r1) * 1.00000095367431641f; // (1 + 2^-20): outward over the roundings
+        if (node == 0) return;
+        slot = parent_inner[node];
+    }
 }
 
 } // namespace rtb

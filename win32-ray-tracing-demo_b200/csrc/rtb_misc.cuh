@@ -1,10 +1,11 @@
 // rtb_misc.cuh -- the non-template kernels of the library (sm_100a): tile-order counting sort, parity hooks
-// (primary rays with traversal recording, ray batches), ray and closest-point queries, the PerformanceTest bounce loop,
-// frame un-sharding.
+// (primary rays with traversal recording, ray batches), ray, closest-point and winding-number queries, the PerformanceTest
+// bounce loop, frame un-sharding.
 // Included by exactly one translation unit (rtb_abi.cu).
 #pragma once
 #include "rtb_kernels.cuh"
 #include "rtb_closest.h"
+#include "rtb_winding.h"
 
 namespace rtb {
 
@@ -388,6 +389,88 @@ k_query_points(const __grid_constant__ DScene S, const __grid_constant__ PointPa
     if (Q.distance) Q.distance[i] = id >= 0 ? sqrtf(best) : -1.0f;
     if (Q.position) { Q.position[3 * i] = q[0]; Q.position[3 * i + 1] = q[1]; Q.position[3 * i + 2] = q[2]; }
     if (Q.normal) { Q.normal[3 * i] = nrm[0]; Q.normal[3 * i + 1] = nrm[1]; Q.normal[3 * i + 2] = nrm[2]; }
+}
+
+// Winding-number queries (rtb_query_winding): w(p) = sum of the TRIANGLES and MESH records' solid angles / 4 pi (include/rtb.h,
+// DESIGN 3f).  The moments are rtb_scene's, not DScene's, so no other kernel's parameters change.
+struct WindingParams
+{
+    long long n;
+    const float *points;
+    const float4 *moments; // rtb_scene::mesh_moments: 4 float4 per node slot, parallel to DScene::mesh_nodes
+    float beta;
+    float *winding;
+    uint8_t *inside;
+};
+
+// one triangle's exact term, fl(Omega * fl(1 / 4 pi))
+__device__ __forceinline__ float windingOf(const float4 *tris, unsigned int idx, const float p[3])
+{
+    const TriData T = loadTri(tris, idx);
+    const float t[9] = {T.q0.x, T.q0.y, T.q0.z, T.q0.w, T.q1.x, T.q1.y, T.q1.z, T.q1.w, T.q2.x};
+    return rtb_winding::solidAngle(p, t) * RTB_WINDING_INV4PI;
+}
+
+// The hierarchy of a MESH record, walked from the root with nothing pruned: per step the child links and both children's
+// moments {N0, c0, r0, N1, c1, r1}; a leaf child adds its exact term, an inner child farther than beta r adds its dipole,
+// any other child is descended into (the first, the second pushed).  w comes in as the earlier records' sum.
+__device__ float meshWinding(const DScene &S, const float4 *moments, unsigned int base, const float p[3], float beta, float w)
+{
+    const float4 *nodes = S.mesh_nodes + 4ull * base, *mom = moments + 4ull * base;
+    int stack[RTB_BVH_STACK];
+    int sp = 0, node = 0;
+    while (true)
+    {
+        const float4 q3 = __ldg(nodes + 4ull * (unsigned int)node + 3);
+        const float4 *m = mom + 4ull * (unsigned int)node;
+        const float4 m0 = __ldg(m), m1 = __ldg(m + 1), m2 = __ldg(m + 2), m3 = __ldg(m + 3);
+        const int ch[2] = {__float_as_int(q3.x), __float_as_int(q3.y)};
+        const float N[2][3] = {{m0.x, m0.y, m0.z}, {m1.w, m2.x, m2.y}};
+        const float c[2][3] = {{m0.w, m1.x, m1.y}, {m2.z, m2.w, m3.x}};
+        const float r[2] = {m1.z, m3.y};
+        const int sides = ch[1] != ch[0] ? 2 : 1; // a one-triangle mesh links its leaf twice
+        bool down[2] = {false, false};
+        for (int s = 0; s < sides; s++)
+        {
+            if (ch[s] < 0) w += windingOf(S.mesh_tris, base + (unsigned int)~ch[s], p);
+            else if (rtb_winding::far(p, c[s], r[s], beta)) w += rtb_winding::dipole(p, N[s], c[s]);
+            else down[s] = true;
+        }
+        if (down[0] && down[1])
+        {
+            stack[sp++] = ch[1];
+            node = ch[0];
+        }
+        else if (down[0]) node = ch[0];
+        else if (down[1]) node = ch[1];
+        else
+        {
+            if (sp == 0) break;
+            node = stack[--sp];
+        }
+    }
+    return w;
+}
+
+__global__ void __launch_bounds__(RTB_CTA_THREADS)
+k_query_winding(const __grid_constant__ DScene S, const __grid_constant__ WindingParams Q)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= Q.n) return;
+    const float p[3] = {__ldg(Q.points + 3 * i), __ldg(Q.points + 3 * i + 1), __ldg(Q.points + 3 * i + 2)};
+    float w = 0.0f;
+    if (!(p[0] == p[0] && p[1] == p[1] && p[2] == p[2])) w = NAN; // a NaN point: NaN / outside, without a walk
+    else
+        for (int j = 0; j < S.n_prims; j++)
+        {
+            const rtb_prim &P = S.prims[j];
+            if (P.type == RTB_PRIM_TRIANGLES)
+                for (int k = 0; k < P.count; k++) w += windingOf(S.loose, (unsigned int)(P.first + k), p);
+            else if (P.type == RTB_PRIM_MESH)
+                w = meshWinding(S, Q.moments, (unsigned int)S.mesh_base[j], p, Q.beta, w);
+        }
+    if (Q.winding) Q.winding[i] = w;
+    if (Q.inside) Q.inside[i] = w > 0.5f ? 1 : 0;
 }
 
 // ---------------------------------------------------------------------------------------------
