@@ -419,6 +419,30 @@ int rtb_scene_mesh_moments(rtb_ctx *ctx, rtb_scene *scene, void *stream);
 int rtb_query_winding(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *points, float beta, float *winding,
                       uint8_t *inside, void *stream);
 
+/* Triangle intersection queries on DEVICE buffers, stream-ordered like rtb_query_points: which of the scene's triangles a
+ * batch of triangles touches, for contact between a deforming body and a scene, cloth against a body, or checking that an
+ * edit or an optimisation step does not make two parts interpenetrate.  tris = [n][12] in the loose_tri format (a, b, c,
+ * normal; the normal is ignored), 16-byte aligned; n <= INT32_MAX.  Records considered: TRIANGLES and MESH records, in prims
+ * order (PLANE, SPHERE and TUNNEL records are ignored); a scene triangle k is (a, fl(a - e1), fl(a - e2)) of its packed record,
+ * with hit id base_id + k, so a triangle inside two overlapping records is reported once per record.
+ * A pair is reported EXACTLY when the two closed triangles share at least one point in exact real arithmetic: touching counts
+ * (a shared vertex, a vertex on the other's face, coplanar triangles that overlap or touch); there is no tolerance.  The one
+ * exception: DEGENERATE triangles, on either side -- three exactly collinear vertices (repeated vertices included) or a
+ * non-finite coordinate -- are never reported.  The decision is csrc/rtb_tritri.h, exact orientation predicates compiled for
+ * host and device; a MESH record prunes its hierarchy by closed boxes and gives what a loop over its triangles gives.
+ *   RTB_QUERY_ANY: hit[n] (uint8, 1-byte aligned, required) = 1 exactly when RTB_QUERY_PAIRS reports a pair for triangle i,
+ *     else 0; pairs and count must be NULL and capacity 0.  A triangle's search stops at its first pair.
+ *   RTB_QUERY_PAIRS: *count (int64, 8-byte aligned, required) is zeroed on the stream, then holds the number of pairs, even
+ *     when it exceeds capacity.  pairs = [capacity][2] int32 (i, hit_id), 8-byte aligned: slots 0 .. min(count, capacity) - 1
+ *     are written and nothing beyond them.  The order is unspecified; the set is deterministic.  capacity = 0 with pairs NULL
+ *     counts only; size the buffer from *count and call again.  hit must be NULL.
+ * Ordering as rtb_query_points; no host synchronisation, no allocation.  Refused with RTB_ERR_INVALID, writing nothing: n < 0 or
+ * above INT32_MAX, capacity < 0, capacity > 0 with pairs NULL, unknown flags, outputs that do not match them, host memory,
+ * memory of another device, a misaligned buffer.  n == 0 launches nothing (PAIRS still zeroes *count).                   */
+enum { RTB_QUERY_PAIRS = 2 };
+int rtb_query_triangles(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *tris, int32_t flags, uint8_t *hit,
+                        int32_t *pairs, int64_t capacity, int64_t *count, void *stream);
+
 /* Replaces the ray loop of the reference's PerformanceTest console benchmark
  * (src/PerformanceTest/main.cpp:29-59 `trace`, 151-162): every ray of the batch [n][6] (HOST) is
  * mirror-reflected off whatever it hits until it reaches a PLANE geometry (the plane closing the tunnel

@@ -26,6 +26,7 @@ PRIM_PLANE, PRIM_SPHERE, PRIM_TRIANGLES, PRIM_TUNNEL, PRIM_MESH = 0, 1, 2, 3, 4 
 MESH_REBUILD, MESH_REFIT = 0, 1  # rtb_scene_mesh_update flags
 CUDA_STREAM_LEGACY = 1  # cudaStreamLegacy
 QUERY_CLOSEST, QUERY_ANY = 0, 1  # rtb_query_rays / rtb_query_points flags
+QUERY_PAIRS = 2  # rtb_query_triangles: every intersecting pair (QUERY_ANY: a flag per triangle)
 
 
 class RtbError(RuntimeError):
@@ -142,7 +143,7 @@ ABI_SYMBOLS = ["rtb_init", "rtb_shutdown", "rtb_last_error", "rtb_abi_version", 
                "rtb_multi_init", "rtb_multi_shutdown", "rtb_multi_count", "rtb_multi_ctx", "rtb_multi_last_error",
                "rtb_multi_scene_upload", "rtb_multi_scene_free", "rtb_multi_scene_upload_bytes", "rtb_multi_render",
                "rtb_multi_scene_mesh_update", "rtb_query_rays", "rtb_query_points",
-               "rtb_scene_mesh_moments", "rtb_query_winding"]
+               "rtb_scene_mesh_moments", "rtb_query_winding", "rtb_query_triangles"]
 
 _cuda = None
 _host = None
@@ -191,6 +192,7 @@ def cuda_lib():
         lib.rtb_query_points.argtypes = [vp, vp, i64, vp, vp, C.c_float, i32, vp, vp, vp, vp, vp, vp]
         lib.rtb_scene_mesh_moments.argtypes = [vp, vp, vp]
         lib.rtb_query_winding.argtypes = [vp, vp, i64, vp, C.c_float, vp, vp, vp]
+        lib.rtb_query_triangles.argtypes = [vp, vp, i64, vp, i32, vp, vp, i64, vp, vp]
         lib.rtb_forget_schedule.argtypes = [vp]
         lib.rtb_device_alloc.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
         lib.rtb_device_free.argtypes = [vp, vp]
@@ -911,6 +913,68 @@ class DeviceScene:
                                                         None if inside else p, p if inside else None, C.c_void_p(stream or 0)),
                         "rtb_query_winding")
         return out
+
+    def intersects(self, tris, stream=None, out=None):
+        """rtb_query_triangles with QUERY_ANY: a torch.bool tensor [m], True where the query triangle shares a point with one
+        of the scene's TRIANGLES or MESH triangles, decided exactly (include/rtb.h; degenerate triangles never intersect).
+        `tris` is a contiguous CUDA float32 tensor [m][12] (a, b, c, normal; the normal is ignored) on the context's device.
+        On the device and ordered on `stream` with no host synchronisation; streams and `out` (a bool tensor [m]) as in
+        query."""
+        import torch
+        tris, dev = self._query_tris(tris, "intersects")
+        m = tris.shape[0]
+        stream, alloc_stream = _query_stream(dev, stream)
+        if out is None:
+            with torch.cuda.stream(alloc_stream):
+                out = torch.empty(m, dtype=torch.bool, device=dev)
+        elif not (isinstance(out, torch.Tensor) and out.device == dev and out.dtype == torch.bool and tuple(out.shape) == (m,)
+                  and out.is_contiguous()):
+            raise RtbError(f"intersects: out must be a contiguous bool tensor [{m}] on {dev}")
+        if m == 0:
+            return out
+        self.ctx._check(self.ctx._lib.rtb_query_triangles(self.ctx._h, self._h, m, C.c_void_p(tris.data_ptr()), QUERY_ANY,
+                                                          C.c_void_p(out.data_ptr()), None, 0, None, C.c_void_p(stream or 0)),
+                        "rtb_query_triangles")
+        return out
+
+    def intersecting_pairs(self, tris, capacity=None, stream=None):
+        """rtb_query_triangles with QUERY_PAIRS: an int64 tensor [P][2] of every (i, hit_id) whose triangles share a point,
+        sorted lexicographically.  `tris` as in intersects.  This reads the pair count back, so it SYNCHRONISES with
+        `stream`; the query runs a second time only when the first buffer of `capacity` pairs (default: m) was too small."""
+        import torch
+        tris, dev = self._query_tris(tris, "intersecting_pairs")
+        m = tris.shape[0]
+        stream, alloc_stream = _query_stream(dev, stream)
+        cap = m if capacity is None else int(capacity)
+        if cap < 0:
+            raise RtbError("intersecting_pairs: capacity must be >= 0")
+        with torch.cuda.stream(alloc_stream):
+            count = torch.empty(1, dtype=torch.int64, device=dev)
+        while True:
+            with torch.cuda.stream(alloc_stream):
+                pairs = torch.empty((cap, 2), dtype=torch.int32, device=dev)
+            self.ctx._check(self.ctx._lib.rtb_query_triangles(self.ctx._h, self._h, m, C.c_void_p(tris.data_ptr()), QUERY_PAIRS,
+                                                              None, C.c_void_p(pairs.data_ptr()) if cap else None, cap,
+                                                              C.c_void_p(count.data_ptr()), C.c_void_p(stream or 0)),
+                            "rtb_query_triangles")
+            alloc_stream.synchronize()
+            total = int(count.cpu()[0])
+            if total <= cap:
+                break
+            cap = total
+        with torch.cuda.stream(alloc_stream):
+            p = pairs[:total].to(torch.int64)
+            p = p[torch.argsort(p[:, 0] * (1 << 32) + p[:, 1])]
+        alloc_stream.synchronize()
+        return p
+
+    def _query_tris(self, tris, what):
+        import torch
+        dev = torch.device("cuda", self.ctx.device)
+        if not (isinstance(tris, torch.Tensor) and tris.device == dev and tris.dtype == torch.float32 and tris.is_contiguous()
+                and tris.dim() == 2 and tris.shape[1] == 12):
+            raise RtbError(f"{what}: tris must be a contiguous float32 tensor [m][12] on {dev}")
+        return tris, dev
 
 
 def _query_stream(dev, stream):

@@ -23,7 +23,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 CUDA_UNITS = ["rtb_abi.cu", "rtb_k_chain.cu", "rtb_k_sm.cu", "rtb_k_oct.cu", "rtb_k_wide.cu", "rtb_k_mc.cu"]
 CUDA_HEADERS = ["rtb_launch.h", "rtb_misc.cuh", "rtb_chain_sm.cuh", "rtb_chain_wide.cuh", "rtb_chain_oct.cuh", "rtb_build_grid.cuh",
                 "rtb_kernels.cuh", "rtb_device.cuh", "rtb_pretest.h", "rtb_sat.h", "rtb_bvh.h", "rtb_build_bvh.cuh", "rtb_closest.h",
-                "rtb_winding.h"]
+                "rtb_winding.h", "rtb_tritri.h"]
 GXX_FLAGS = ["-O2", "-std=c++17", "-fopenmp", "-ffp-contract=off", "-fPIC", "-shared", "-Wall"]
 
 

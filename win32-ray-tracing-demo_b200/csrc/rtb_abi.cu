@@ -2685,7 +2685,7 @@ static void launchQuery(const rtb_scene *scene, const QueryParams &Q, bool any, 
     else k_query_rays<false, false><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
 }
 
-// A caller's buffer for rtb_query_rays / rtb_query_points / rtb_query_winding: memory of the context's device or managed memory, `align`-byte aligned
+// A caller's buffer for rtb_query_rays / rtb_query_points / rtb_query_winding / rtb_query_triangles: memory of the context's device or managed memory, `align`-byte aligned
 static bool deviceBuffer(const rtb_ctx *ctx, const void *p, uintptr_t align)
 {
     cudaPointerAttributes attr;
@@ -2695,7 +2695,7 @@ static bool deviceBuffer(const rtb_ctx *ctx, const void *p, uintptr_t align)
     return attr.type == cudaMemoryTypeManaged || (attr.type == cudaMemoryTypeDevice && attr.device == ctx->device);
 }
 
-// The part rtb_query_rays, rtb_query_points and rtb_query_winding share.  Before the launch (queryBegin): the buffer checks -- the input array
+// The part rtb_query_rays, rtb_query_points, rtb_query_winding and rtb_query_triangles share.  Before the launch (queryBegin): the buffer checks -- the input array
 // `in` (required) and the optional bound and outputs `bufs` -- and the ordering of the caller's stream behind the scene's
 // upload / updates and behind the last query on another stream.  After it (queryEnd): query_use recorded on that stream.
 // Every check comes before anything is enqueued.
@@ -2789,6 +2789,36 @@ extern "C" int rtb_query_winding(rtb_ctx *ctx, const rtb_scene *scene, int64_t n
     Q.n = (long long)n; Q.points = points; Q.moments = scene->mesh_moments; Q.beta = beta;
     Q.winding = winding; Q.inside = inside;
     k_query_winding<<<(unsigned int)((Q.n + RTB_CTA_THREADS - 1) / RTB_CTA_THREADS), RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+    return queryEnd(ctx, scene, st);
+}
+
+extern "C" int rtb_query_triangles(rtb_ctx *ctx, const rtb_scene *scene, int64_t n, const float *tris, int32_t flags, uint8_t *hit,
+                                   int32_t *pairs, int64_t capacity, int64_t *count, void *stream)
+{
+    if (!ctx || !scene || n < 0 || n > INT32_MAX) return fail(ctx, RTB_ERR_INVALID, "rtb_query_triangles: bad argument (n must be in [0, INT32_MAX])");
+    if (flags != RTB_QUERY_ANY && flags != RTB_QUERY_PAIRS) return fail(ctx, RTB_ERR_INVALID, "rtb_query_triangles: unknown flags");
+    const bool any = flags == RTB_QUERY_ANY;
+    if (capacity < 0 || (capacity > 0 && !pairs)) return fail(ctx, RTB_ERR_INVALID, "rtb_query_triangles: capacity < 0, or capacity > 0 without pairs");
+    if (any ? (!hit || pairs || count || capacity) : (hit || !count))
+        return fail(ctx, RTB_ERR_INVALID, "rtb_query_triangles: the outputs do not match the flags (ANY: hit only; PAIRS: count and pairs, no hit)");
+    if (n == 0 && any) return RTB_OK;
+    const void *bufs[6] = {hit, pairs, n ? count : nullptr, nullptr, nullptr, nullptr};
+    const uintptr_t align[6] = {1, 8, 8, 1, 1, 1};
+    cudaStream_t st;
+    // n == 0 in PAIRS mode reads no triangles but still defines *count: the count stands in for the input
+    const int rc = n ? queryBegin(ctx, scene, "rtb_query_triangles", "tris", tris, 16, bufs, align, "the outputs", stream, st)
+                     : queryBegin(ctx, scene, "rtb_query_triangles", "count", count, 8, bufs, align, "the outputs", stream, st);
+    if (rc != RTB_OK) return rc;
+    if (!any) CUDA_TRY(ctx, cudaMemsetAsync(count, 0, sizeof(int64_t), st));
+    if (n > 0)
+    {
+        TriQueryParams Q = {};
+        Q.n = (long long)n; Q.tris = tris; Q.hit = hit; Q.pairs = reinterpret_cast<int2 *>(pairs); Q.capacity = (long long)capacity;
+        Q.count = reinterpret_cast<unsigned long long *>(count);
+        const unsigned int blocks = (unsigned int)((Q.n + RTB_CTA_THREADS - 1) / RTB_CTA_THREADS);
+        if (any) k_query_triangles<true><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+        else k_query_triangles<false><<<blocks, RTB_CTA_THREADS, 0, st>>>(scene->d, Q);
+    }
     return queryEnd(ctx, scene, st);
 }
 

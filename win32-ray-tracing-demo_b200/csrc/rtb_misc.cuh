@@ -1,11 +1,12 @@
 // rtb_misc.cuh -- the non-template kernels of the library (sm_100a): tile-order counting sort, parity hooks
-// (primary rays with traversal recording, ray batches), ray, closest-point and winding-number queries, the PerformanceTest
+// (primary rays with traversal recording, ray batches), ray, closest-point, winding-number and triangle queries, the PerformanceTest
 // bounce loop, frame un-sharding.
 // Included by exactly one translation unit (rtb_abi.cu).
 #pragma once
 #include "rtb_kernels.cuh"
 #include "rtb_closest.h"
 #include "rtb_winding.h"
+#include "rtb_tritri.h"
 
 namespace rtb {
 
@@ -471,6 +472,117 @@ k_query_winding(const __grid_constant__ DScene S, const __grid_constant__ Windin
         }
     if (Q.winding) Q.winding[i] = w;
     if (Q.inside) Q.inside[i] = w > 0.5f ? 1 : 0;
+}
+
+// Triangle queries (rtb_query_triangles): which TRIANGLES and MESH triangles each query triangle shares a point with, decided
+// exactly by rtb_tritri.h (include/rtb.h, DESIGN 3g).  ANY: hit[i]; otherwise every pair (i, hit_id) is counted in *count and
+// stored while the count is below capacity.
+struct TriQueryParams
+{
+    long long n;
+    const float *tris; // [n][12] a, b, c, normal; 16-byte aligned
+    uint8_t *hit;
+    int2 *pairs;
+    long long capacity;
+    unsigned long long *count;
+};
+
+// One pair, appended with one atomic per group of lanes that report together.
+__device__ __forceinline__ void appendPair(const TriQueryParams &Q, int i, int id)
+{
+    const unsigned int mask = __activemask();
+    const int lane = threadIdx.x & 31, leader = __ffs(mask) - 1;
+    unsigned long long at = 0;
+    if (lane == leader) at = atomicAdd(Q.count, (unsigned long long)__popc(mask));
+    at = __shfl_sync(mask, at, leader) + (unsigned long long)__popc(mask & ((1u << lane) - 1u));
+    if (at < (unsigned long long)Q.capacity) Q.pairs[at] = make_int2(i, id);
+}
+
+// the scene triangle at packed position idx as (a, fl(a - e1), fl(a - e2)), and whether it meets the query triangle p
+__device__ __forceinline__ bool triMeets(const float4 *tris, unsigned int idx, const float p[9], const float lo[3], const float hi[3])
+{
+    const TriData T = loadTri(tris, idx);
+    const float t[9] = {T.q0.x, T.q0.y, T.q0.z, T.q0.x - T.q0.w, T.q0.y - T.q1.x, T.q0.z - T.q1.y,
+                        T.q0.x - T.q1.z, T.q0.y - T.q1.w, T.q0.z - T.q2.x};
+    float tlo[3], thi[3];
+    rtb_tritri::box(t, tlo, thi);
+    return rtb_tritri::boxesOverlap(lo, hi, tlo, thi) && rtb_tritri::meets(p, t);
+}
+
+// The hierarchy of a MESH record, walked from the root with meshClosest's node loads: both children's boxes per step against
+// the query triangle's box, an overlapping leaf tested, overlapping inner children descended (the first, the second pushed).
+// ANY: returns true at the first pair.
+template <bool ANY>
+__device__ bool meshTriangles(const DScene &S, const TriQueryParams &Q, unsigned int base, int baseId, int i, const float p[9],
+                              const float lo[3], const float hi[3])
+{
+    const float4 *nodes = S.mesh_nodes + 4ull * base;
+    int stack[RTB_BVH_STACK];
+    int sp = 0, node = 0;
+    while (true)
+    {
+        const float4 *q = nodes + 4ull * (unsigned int)node;
+        const float4 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2), q3 = __ldg(q + 3);
+        const float lo0[3] = {q0.x, q0.y, q0.z}, lo1[3] = {q0.w, q1.x, q1.y};
+        const float hi0[3] = {q1.z, q1.w, q2.x}, hi1[3] = {q2.y, q2.z, q2.w};
+        const int c[2] = {__float_as_int(q3.x), __float_as_int(q3.y)};
+        const int sides = c[1] != c[0] ? 2 : 1; // a one-triangle mesh links its leaf twice
+        const bool o[2] = {rtb_tritri::boxesOverlap(lo, hi, lo0, hi0), sides == 2 && rtb_tritri::boxesOverlap(lo, hi, lo1, hi1)};
+        for (int s = 0; s < sides; s++)
+            if (c[s] < 0 && o[s] && triMeets(S.mesh_tris, base + (unsigned int)~c[s], p, lo, hi))
+            {
+                if (ANY) return true;
+                appendPair(Q, i, baseId + (int)__ldg(S.mesh_order + base + (unsigned int)~c[s]));
+            }
+        const bool in0 = c[0] >= 0 && o[0], in1 = c[1] >= 0 && o[1];
+        if (in0 && in1)
+        {
+            stack[sp++] = c[1];
+            node = c[0];
+        }
+        else if (in0) node = c[0];
+        else if (in1) node = c[1];
+        else
+        {
+            if (sp == 0) break;
+            node = stack[--sp];
+        }
+    }
+    return false;
+}
+
+template <bool ANY>
+__global__ void __launch_bounds__(RTB_CTA_THREADS)
+k_query_triangles(const __grid_constant__ DScene S, const __grid_constant__ TriQueryParams Q)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= Q.n) return;
+    const float4 *t4 = reinterpret_cast<const float4 *>(Q.tris) + 3 * i;
+    const float4 a = __ldg(t4), b = __ldg(t4 + 1), c = __ldg(t4 + 2);
+    const float p[9] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x};
+    bool found = false;
+    if (!rtb_tritri::degenerate(p))
+    {
+        float lo[3], hi[3];
+        rtb_tritri::box(p, lo, hi);
+        for (int j = 0; j < S.n_prims && !(ANY && found); j++)
+        {
+            const rtb_prim &P = S.prims[j];
+            if (P.type == RTB_PRIM_TRIANGLES)
+            {
+                for (int k = 0; k < P.count; k++)
+                    if (triMeets(S.loose, (unsigned int)(P.first + k), p, lo, hi))
+                    {
+                        found = true;
+                        if (ANY) break;
+                        appendPair(Q, (int)i, P.base_id + k);
+                    }
+            }
+            else if (P.type == RTB_PRIM_MESH)
+                found = meshTriangles<ANY>(S, Q, (unsigned int)S.mesh_base[j], P.base_id, (int)i, p, lo, hi) || found;
+        }
+    }
+    if (ANY) Q.hit[i] = found ? 1 : 0;
 }
 
 // ---------------------------------------------------------------------------------------------
